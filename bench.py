@@ -15,7 +15,7 @@ N > 1: every rank runs its own sequence (frame sharding, no data-path collective
            frames and D2H of the int8 partition vectors inside the timed region.
 `roofline`: the conv kernel class that dominates the step, algorithmic FLOPs / CUDA-event time of its launches over a
            second pass of the same K steps (per-launch event pairs; `value` is timed without them), against the
-           measured bf16 peak in MEASURED_PEAKS.json.
+           measured bf16 peak, see peaks().
 `cpu_baseline`: the oracle port of the reference's CPU path (PyTorch CPU fp32 nets + NumPy post-process/decode),
            timed on this host on a bounded sample of the same workload (rank 0, N=1 only).
 `gpu_baseline`: the only GPU implementation the reference has -- its PyTorch modules under torch/cuDNN
@@ -29,6 +29,9 @@ N > 1: every rank runs its own sequence (frame sharding, no data-path collective
 `--impl torch-cuda`: times the torch/cuDNN arm alone (same metric/config).
 `--workload 4k30`: BASELINE configs[2] -- ONE synthetic 3840x2160 30-frame sequence strong-scaled over the N ranks by
            frame sharding (Map2Partition.py:389-412 makes the gather a concatenation), see fourk_main().
+`--dump-outputs DIR`: after the timed steps, rank 0 writes what the last timed step returned (the int8 PartitionMat
+           vectors of every component and QP) as DIR/<comp>_QP<qp>.npy, see dump_outputs().  The inputs are seeded, so two
+           builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -64,12 +67,15 @@ def workload_config(engine=None):
 
 
 def peaks():
+    """Roofline denominators: the B200 peaks measured for this project (BASELINE.md section 2), unless a
+    MEASURED_PEAKS.json beside this file holds peaks measured on the card at hand."""
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
         d = json.load(open(p))
         return {"hbm_gbs": d["hbm_gbs"], "bf16_burst": d["bf16_tflops"], "bf16_sustained": d["bf16_tflops_sustained"],
                 "src": "measured (MEASURED_PEAKS.json)"}
-    return {"hbm_gbs": 6650.0, "bf16_burst": 1590.0, "bf16_sustained": 1400.0, "src": "fallback (B200_PROFILING.md)"}
+    return {"hbm_gbs": 6446.6, "bf16_burst": 1660.1, "bf16_sustained": 1413.7,
+            "src": "measured on a B200, power limit not recorded (BASELINE.md section 2)"}
 
 
 class ClockSampler:
@@ -133,6 +139,26 @@ def make_frames(seed, width=WIDTH, height=HEIGHT, frames=FRAMES):
     us = np.stack([np.roll(u[k], 4 * i, axis=1) for i, k in enumerate(idx)])
     vs = np.stack([np.roll(v[k], 4 * i, axis=1) for i, k in enumerate(idx)])
     return ys, us, vs
+
+
+# values kept per output by dump_outputs: 8 outputs x 2^20 float32 = 32 MB per dump (a step returns 51.6 M int8 values)
+DUMP_SAMPLE = 1 << 20
+
+
+def dump_outputs(out_dir, results, sample=DUMP_SAMPLE):
+    """Write {(comp, qp): int8 tensor [F, per-frame values]} as out_dir/<comp>_QP<qp>.npy, float32, flattened.  An output
+    longer than `sample` is reduced to the values at `sample` sorted positions drawn with a fixed seed (the same positions
+    for every output of that length, in every run).  Returns {name: number of values written}."""
+    os.makedirs(out_dir, exist_ok=True)
+    written = {}
+    for (comp, qp), vals in sorted(results.items()):
+        a = vals.cpu().numpy().reshape(-1)
+        if a.size > sample:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, size=sample, replace=False))]
+        name = "%s_QP%d" % (comp, qp)
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
+        written[name] = int(a.size)
+    return written
 
 
 def kernel_source_sha():
@@ -513,7 +539,14 @@ def main():
     ap.add_argument("--chunk", type=int, default=4800)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-profile", action="store_true")
+    ap.add_argument("--dump-outputs", type=str, default=None, metavar="DIR",
+                    help="write what the last timed step computed as DIR/<comp>_QP<qp>.npy (float32, a fixed seeded "
+                         "sample of %d values per output)" % DUMP_SAMPLE)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "1080p10"):
+        ap.error("--dump-outputs is implemented for --impl b200 --workload 1080p10")
     if args.impl == "reference":
         return reference_main(args)
     if args.impl == "torch-cuda":
@@ -557,17 +590,19 @@ def main():
         torch.cuda.synchronize()
 
     def timed(fn, steps):
+        """(ms of `steps` calls of fn, what the last call returned)"""
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         barrier()
         e0.record()
-        for _ in range(steps):
+        for _ in range(steps - 1):
             fn()
+        last = fn()
         e1.record()
         barrier()
         ms = torch.tensor([e0.elapsed_time(e1)], device="cuda")
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item())
+        return float(ms.item()), last
 
     for _ in range(args.warmup):
         step_device()
@@ -577,20 +612,22 @@ def main():
     if rank == 0:
         sampler.start()
     l0 = h.launch_count()
-    ms = timed(step_device, args.steps)                 # `value`: no per-launch events in the stream
+    ms, last = timed(step_device, args.steps)           # `value`: no per-launch events in the stream
     launches = h.launch_count() - l0
     clocks = sampler.stop() if rank == 0 else None
+    dumped = dump_outputs(args.dump_outputs, last) if args.dump_outputs and rank == 0 else None
+    del last
     # roofline pass: the same K steps again with a CUDA-event pair around every launch (the events sit between the
     # kernels, which switches off the programmatic-dependent-launch overlap, hence a separate pass)
     prof, ms_prof = {}, None
     if not args.no_profile:
         h.profile(2)
-        ms_prof = timed(step_device, args.steps)
+        ms_prof, _ = timed(step_device, args.steps)
         prof = h.profile_read()
         h.profile(0)
 
     step_e2e()
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
     decode_report = pp.counts() if rank == 0 else None
     text_leg = None
     if rank == 0 and not args.no_text_write:
@@ -659,6 +696,10 @@ def main():
         text_leg["ctu_per_s_text_only"] = units / sec
         text_leg["ctu_per_s_e2e_plus_text"] = units / (ms_e2e * 1e-3 / args.steps + sec)
         out["text_write"] = text_leg
+    if dumped:
+        out["dump_outputs"] = {"dir": args.dump_outputs, "values": dumped, "dtype": "float32",
+                               "sample": "int8 PartitionMat vectors of the last timed step, flattened; outputs longer than "
+                                         "%d values sampled at fixed seeded positions" % DUMP_SAMPLE}
     if world == 1 and not args.no_gpu_baseline:
         pp.close()
         torch.cuda.empty_cache()
