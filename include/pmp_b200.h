@@ -51,7 +51,8 @@ enum pmp_in_dtype { PMP_IN_U8 = 0, PMP_IN_F32 = 1 };
 int pmp_version(void);
 const char *pmp_last_error(void);
 
-/* Lifetime.  pmp_create binds to `device`, creates no streams of its own.  A new handle runs PMP_ENGINE_TC / PMP_TC_FP16. */
+/* Lifetime.  pmp_create binds to `device` and creates no streams; pmp_predict_host creates two streams and pinned staging
+ * buffers on its first call, which pmp_destroy frees.  A new handle runs PMP_ENGINE_TC / PMP_TC_FP16. */
 int pmp_create(int device, pmp_handle **out);
 void pmp_destroy(pmp_handle *h);
 int pmp_set_engine(pmp_handle *h, int engine, int tc_dtype);
@@ -79,6 +80,13 @@ int pmp_profile_read(pmp_handle *h, int idx, char *name, int name_len, double *m
 int pmp_weights_create(pmp_handle *h, int net, const float *const *tensors_host, const int64_t *numel,
                        int n_tensors, int *wset);
 int pmp_weights_destroy(pmp_handle *h, int wset);
+/* Same from an exported weight file (.pmpw, python -m pmp_vvc_tip2023_b200.export_weights), read on the host: a 64-byte
+ * header ("PMPW0001", int32 net kind, int32 tensor count, int64 total floats, uint64 FNV-1a-64 of everything after the
+ * header), one record per tensor (int32 name length, name, int32 ndim, int32 dims[ndim]), zero padding to a multiple of
+ * 64 bytes, then the fp32 data in record order, all little-endian.  Every field is checked against the library's own
+ * parameter table; any mismatch returns PMP_ERR_ARG, creates no weight set and names the path and the first field that
+ * failed.  *net_out (may be NULL) receives the net kind, *wset the weight-set id. */
+int pmp_weights_load(pmp_handle *h, const char *path, int *net_out, int *wset);
 
 /* ---- nets ------------------------------------------------------------------------------
  * pmp_forward_q      == Luma_Q_Net.forward / Chroma_Q_Net.forward      (Model_QBD.py:78-98,:176-196)
@@ -147,6 +155,27 @@ int pmp_cut_blocks(pmp_handle *h, const void *y, const void *u, const void *v, i
 int pmp_run_component(pmp_handle *h, int wset_q, int wset_msbd, int luma, const uint8_t *blocks, int frames,
                       int bh, int bw, int chunk, int8_t *out, float *qt_raw, float *bt, float *dire,
                       uint32_t *flags, void *stream);
+
+/* pmp_predict_host == the per-QP body of Inference_QBD.py:190-241 from host planes to host PartitionMat vectors
+ * (get_sequence_partition_for_VTM order, Map2Partition.py:389-412), for callers without CUDA of their own.
+ * wsets: luma Q, luma MSBD, chroma Q, chroma MSBD weight sets of one QP; -1,-1 skips that component.
+ * y [F][H][pitch_y], u/v [F][H/2][pitch_c]: HOST pointers (pageable or pinned); pitches in bytes, 0 = dense; sample_bytes
+ * as in pmp_cut_blocks (u and v may be NULL when chroma is skipped).  luma_out / chroma_out: HOST, frames *
+ * pmp_frame_values(H/64, W/64) int8 each, the text file's values and the .bin payload.  Width or height below 64 means
+ * zero blocks: PMP_OK, nothing written.
+ * Frames are processed in windows of max(1, chunk / blocks-per-frame) whole frames (chunk <= 0: 4800), staged through
+ * library-owned pinned buffers; the next window's upload and the previous one's download overlap the current window's
+ * kernels.  Synchronous: returns when both outputs are in host memory.
+ * report (may be NULL): decode-flag counts of this call summed over both components (flags of pmp_map2partition;
+ * near_threshold = bits 1..3, tight = bits 4..6) and the fp16 saturation events of this call (the sticky counter of
+ * pmp_saturation_count is not reset).  Saturation events make the call return PMP_ERR_STATE: rerun with PMP_TC_BF16
+ * (Inference_QBD.py:192-194 of this package refuses the same way). */
+typedef struct pmp_report {
+    long long blocks, near_tie_blocks, near_threshold_blocks, near_threshold_blocks_tight, fp16_saturation_events;
+} pmp_report;
+int pmp_predict_host(pmp_handle *h, const int wsets[4], const void *y, const void *u, const void *v, int sample_bytes,
+                     int64_t pitch_y, int64_t pitch_c, int frames, int width, int height, int chunk, int8_t *luma_out,
+                     int8_t *chroma_out, pmp_report *report);
 
 /* Self-test of the TC conv engine against the SIMT engine on random data (GPU).  Returns 0 and the
  * max-abs error in *max_err, or an error.  flags: bit0 ReLU, bit1 identity residual, bit2 attention product,

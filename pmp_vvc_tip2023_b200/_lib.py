@@ -33,6 +33,9 @@ SIGNATURES = {
                                  _P(ctypes.c_double), _P(ctypes.c_double)]),
     "pmp_weights_create": (c_int, [c_void_p, c_int, _P(c_void_p), _P(c_int64), c_int, _P(c_int)]),
     "pmp_weights_destroy": (c_int, [c_void_p, c_int]),
+    "pmp_weights_load": (c_int, [c_void_p, c_char_p, _P(c_int), _P(c_int)]),
+    "pmp_predict_host": (c_int, [c_void_p, _P(c_int), c_void_p, c_void_p, c_void_p, c_int, c_int64, c_int64, c_int, c_int,
+                                 c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "pmp_forward_q": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "pmp_forward_msbd": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p,
                                  c_void_p]),
@@ -65,6 +68,15 @@ _lock = threading.Lock()
 
 class PmpError(RuntimeError):
     pass
+
+
+class Report(ctypes.Structure):
+    """struct pmp_report (pmp_predict_host)."""
+    _fields_ = [(k, ctypes.c_longlong) for k in ("blocks", "near_tie_blocks", "near_threshold_blocks",
+                                                 "near_threshold_blocks_tight", "fp16_saturation_events")]
+
+    def as_dict(self):
+        return {k: int(getattr(self, k)) for k, _ in self._fields_}
 
 
 def lib():
@@ -170,3 +182,41 @@ class Handle:
 
     def weights_destroy(self, wset):
         check(lib().pmp_weights_destroy(self._h, wset))
+
+    def weights_load(self, path):
+        """An exported .pmpw file (export_weights.py) -> (net kind, weight-set id)."""
+        net, wset = c_int(), c_int()
+        check(lib().pmp_weights_load(self._h, os.fsencode(path), ctypes.byref(net), ctypes.byref(wset)))
+        return net.value, wset.value
+
+    # ---- host path ----------------------------------------------------------------------------
+    def predict_host(self, wsets, y, u, v, chunk=0, outs=(None, None), report=None):
+        """pmp_predict_host.  wsets: (luma Q, luma MSBD, chroma Q, chroma MSBD), -1, -1 skips a component.
+        y [F,H,W], u/v [F,H/2,W/2]: host numpy arrays (uint8, or uint16 holding 10-bit samples) or CPU tensors; rows may
+        be padded (a view of the first W columns of wider rows).  outs: (luma, chroma) host buffers of
+        F * pmp_frame_values(H/64, W/64) int8 (numpy arrays or pinned tensors), None = allocate.  Returns the two
+        outputs as int8 [F, per] (None for a skipped component); `report` (a Report) receives the decode report."""
+        import numpy as np
+
+        y, u, v = (a.numpy() if hasattr(a, "data_ptr") else a for a in (y, u, v))
+
+        def plane(a):
+            if a is None:
+                return None, 0
+            assert a.ndim == 3 and a.strides[2] == a.itemsize and a.strides[0] == a.shape[1] * a.strides[1]
+            return c_void_p(a.ctypes.data), a.strides[1]
+
+        f, hgt, wid = y.shape
+        per = int(lib().pmp_frame_values(hgt // 64, wid // 64))
+        res = []
+        for i, o in enumerate(outs):
+            if wsets[2 * i] == -1 and wsets[2 * i + 1] == -1:
+                res.append(None)
+            else:
+                res.append(np.empty((f, per), np.int8) if o is None else o)
+        ptr = [None if o is None else c_void_p(o.data_ptr() if hasattr(o, "data_ptr") else o.ctypes.data) for o in res]
+        (py, sy), (pu, sc), (pv, _) = plane(y), plane(u), plane(v)
+        report = Report() if report is None else report
+        check(lib().pmp_predict_host(self._h, (c_int * 4)(*wsets), py, pu, pv, y.itemsize, sy, sc, f, wid, hgt, int(chunk),
+                                     ptr[0], ptr[1], ctypes.byref(report)))
+        return res

@@ -6,6 +6,11 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libpmp_b200.so")
 SOURCES = ["api.cu", "nets.cu", "decode.cu", "conv_simt.cu", "conv_tc.cu"]
+# host-level entry points (pmp_weights_load, pmp_predict_host) on top of the core; their pmp_destroy releases the host
+# staging and then runs csrc/api.cu's, which is compiled under another name for that
+HOST = os.path.join(HERE, "host")
+HOST_SOURCES = ["host_api.cu"]
+SOURCE_DEFINES = {"api.cu": ["-Dpmp_destroy=pmp_destroy_core"]}
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--use_fast_math=false"]
 
@@ -21,7 +26,8 @@ def stale():
     if not os.path.exists(LIB):
         return True
     t = os.path.getmtime(LIB)
-    deps = [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(HERE, "..", "include", "pmp_b200.h")]
+    deps = [os.path.join(d, f) for d in (CSRC, HOST) for f in os.listdir(d)] + \
+        [os.path.join(HERE, "..", "include", "pmp_b200.h")]
     return any(os.path.getmtime(d) > t for d in deps if os.path.exists(d))
 
 
@@ -33,10 +39,10 @@ def build(force=False, verbose=False):
     procs = []
     os.makedirs(os.path.join(HERE, "build"), exist_ok=True)
     flags = [f for f in NVCC_FLAGS if not f.startswith("--use_fast_math")]
-    for src in SOURCES:
+    for d, src in [(CSRC, s) for s in SOURCES] + [(HOST, s) for s in HOST_SOURCES]:
         obj = os.path.join(HERE, "build", src.replace(".cu", ".o"))
         objs.append(obj)
-        cmd = [_nvcc()] + flags + ["-c", os.path.join(CSRC, src), "-o", obj]
+        cmd = [_nvcc()] + flags + SOURCE_DEFINES.get(src, []) + ["-c", os.path.join(d, src), "-o", obj]
         if verbose:
             cmd += ["-Xptxas", "-v"]
         procs.append((src, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))
@@ -51,6 +57,19 @@ def build(force=False, verbose=False):
     if r.returncode != 0:
         raise RuntimeError("link failed:\n%s" % r.stdout)
     return LIB
+
+
+def build_native_tool(exe):
+    """Compile tools/native/pmp_predict.cpp (C++11, the C header and libpmp_b200.so only) into `exe` with g++, the host
+    compiler nvcc itself uses; the executable finds the in-tree library through its rpath."""
+    root = os.path.dirname(HERE)
+    cmd = [os.environ.get("CXX", "g++"), "-std=c++11", "-O2", "-Wall", "-I" + os.path.join(root, "include"),
+           os.path.join(root, "tools", "native", "pmp_predict.cpp"), "-o", exe, "-L" + HERE, "-lpmp_b200",
+           "-Wl,-rpath," + HERE]
+    r = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
+    if r.returncode != 0:
+        raise RuntimeError("%s failed:\n%s" % (" ".join(cmd), r.stdout))
+    return exe
 
 
 if __name__ == "__main__":

@@ -11,7 +11,7 @@ import numpy as np
 import torch
 
 from . import _lib, ops, synth, weights
-from .netspec import QPS, param_spec
+from .netspec import QPS
 
 COMPS = ("Luma", "Chroma")
 
@@ -56,17 +56,7 @@ class PartitionPredictor:
         out = []
         for kind, sd in (("Q", sd_q), ("MSBD", sd_bd)):
             net = "%s_%s" % (comp, kind)
-            sd = weights.remove_prefix(dict(sd), "module.")
-            tensors = []
-            for name, shape in param_spec(net):
-                if name not in sd:
-                    raise KeyError("%s: missing parameter %s" % (net, name))
-                t = sd[name]
-                t = t.detach().cpu().numpy() if hasattr(t, "detach") else np.asarray(t)
-                if tuple(t.shape) != tuple(shape):
-                    raise ValueError("%s: %s has shape %s, expected %s" % (net, name, tuple(t.shape), tuple(shape)))
-                tensors.append(np.ascontiguousarray(t, dtype=np.float32))
-            out.append(self.handle.weights_create(net, tensors))
+            out.append(self.handle.weights_create(net, [a for _, a in weights.ordered_tensors(net, sd)]))
         old = self._wsets.pop((comp, qp), None)
         if old:
             for w in old:
@@ -79,15 +69,7 @@ class PartitionPredictor:
         in this repo's mount) -- for benchmarking/tests only."""
         for comp in comps:
             for qp in qps:
-                sd_q = weights.load_reference_pkl(os.path.join(model_dir, "%s_Q_%d.pkl" % (comp, qp)))
-                bd_path = os.path.join(model_dir, "%s_BD_%d.pkl" % (comp, qp))
-                if os.path.exists(bd_path):
-                    sd_bd = weights.load_reference_pkl(bd_path)
-                elif missing_bd == "seeded":
-                    sd_bd = synth.seeded_state_dict(comp + "_MSBD", 1000 + qp + (0 if comp == "Luma" else 500))
-                else:
-                    raise FileNotFoundError(bd_path)
-                self.load_state_dicts(comp, qp, sd_q, sd_bd)
+                self.load_state_dicts(comp, qp, *weights.reference_state_dicts(model_dir, comp, qp, missing_bd))
 
     def load_seeded(self, comps=COMPS, qps=QPS, seed=0):
         for comp in comps:
