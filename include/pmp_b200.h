@@ -34,7 +34,8 @@ enum pmp_status {
     PMP_ERR_CUDA = -2,     /* CUDA runtime/driver error (message has the detail) */
     PMP_ERR_NO_DEVICE = -3,
     PMP_ERR_STATE = -4,    /* unknown weight set, wrong net kind ... */
-    PMP_ERR_UNSUPPORTED = -5
+    PMP_ERR_UNSUPPORTED = -5,
+    PMP_ERR_ABORTED = -6   /* a callback of pmp_predict_stream returned non-zero (message names it and its value) */
 };
 
 /* Net kinds: Model_QBD.py:59 Luma_Q_Net, :100 Luma_MSBD_Net, :157 Chroma_Q_Net, :198 Chroma_MSBD_Net */
@@ -51,8 +52,8 @@ enum pmp_in_dtype { PMP_IN_U8 = 0, PMP_IN_F32 = 1 };
 int pmp_version(void);
 const char *pmp_last_error(void);
 
-/* Lifetime.  pmp_create binds to `device` and creates no streams; pmp_predict_host creates two streams and pinned staging
- * buffers on its first call, which pmp_destroy frees.  A new handle runs PMP_ENGINE_TC / PMP_TC_FP16. */
+/* Lifetime.  pmp_create binds to `device` and creates no streams; pmp_predict_host / pmp_predict_stream create two
+ * streams and pinned staging buffers on their first call, which pmp_destroy frees.  A new handle runs PMP_ENGINE_TC / PMP_TC_FP16. */
 int pmp_create(int device, pmp_handle **out);
 void pmp_destroy(pmp_handle *h);
 int pmp_set_engine(pmp_handle *h, int engine, int tc_dtype);
@@ -138,6 +139,13 @@ int64_t pmp_frame_values(int bh, int bw);
  * receives the byte count (synchronises the stream). */
 int pmp_format_text(pmp_handle *h, const int8_t *values, int64_t n, char *text, int64_t *n_bytes_host,
                     void *stream);
+/* pmp_format_texts: the same text for m (1..8) vectors in ONE launch, byte-identical to pmp_format_text per vector, and
+ * without a synchronisation.  values[i] (n[i] int8 in {-1,0,1,2,3}, 0 <= n[i] <= 2^30), text[i] (capacity >= 3*n[i])
+ * and n_bytes (int64[m]): DEVICE pointers, held in host arrays; n: host.  n_bytes[i] is valid when `stream` reaches
+ * this point.  A single-pass scan with per-tile status words that belong to the handle: launches of one handle must not
+ * overlap on different streams.  The first launch of a larger total than before allocates (synchronising the device). */
+int pmp_format_texts(pmp_handle *h, int m, const int8_t *const *values, const int64_t *n, char *const *text,
+                     int64_t *n_bytes, void *stream);
 
 /* ---- input prep ----------------------------------------------------------------------------
  * pmp_cut_blocks == Inference_QBD.output_block_yuv + the chroma input assembly
@@ -176,6 +184,41 @@ typedef struct pmp_report {
 int pmp_predict_host(pmp_handle *h, const int wsets[4], const void *y, const void *u, const void *v, int sample_bytes,
                      int64_t pitch_y, int64_t pitch_c, int frames, int width, int height, int chunk, int8_t *luma_out,
                      int8_t *chroma_out, pmp_report *report);
+
+/* pmp_predict_stream: a sequence of any length from frames to PartitionMat data in bounded memory, for every QP of an
+ * encoder run at once (the whole of Inference_QBD.py:190-241 plus the text of Map2Partition.py:405-412).
+ * wsets: [n_qps][4], each row as pmp_predict_host's (n_qps 1..4; -1,-1 skips a component of that QP, not both).
+ * Frames are processed in windows of window_frames whole frames (<= 0: max(1, 4800 / blocks per frame)).
+ *   read(user, first_frame, frames, y, u, v) fills frames [first_frame, first_frame + frames) as dense planes straight
+ *     into library-owned page-locked memory: y [frames][H][W], u/v [frames][H/2][W/2], sample_bytes per sample; u and v
+ *     are NULL when every QP skips chroma.
+ *   write(user, w) is called once per window, in frame order, on the calling thread, while the GPU computes the next
+ *     window.  w->values[q][c] (c: 0 luma, 1 chroma) holds w->n_values[q][c] = frames * pmp_frame_values(H/64, W/64)
+ *     int8 with PMP_OUT_VALUES; w->text[q][c] holds w->text_bytes[q][c] bytes of file text with PMP_OUT_TEXT.  Pointers
+ *     of a skipped component or an output not asked for are NULL (counts 0).  All are valid only during the callback.
+ *     w->report counts this window only: decode flags of all its results and its fp16 saturation events.
+ * outputs: PMP_OUT_VALUES, PMP_OUT_TEXT or both.  Window k+1 is read and uploaded and window k-1 downloaded and written
+ * while window k computes; each window is cut into blocks once for all its QPs and components, and its texts are
+ * formatted in one launch.  The host waits only on events of finished windows.  Page-locked and device staging scale
+ * with window_frames, not frames; the handle owns them and pmp_destroy frees them.
+ * A non-zero return of either callback stops the call with PMP_ERR_ABORTED.  A window with fp16 saturation events is
+ * still written; the call then stops with PMP_ERR_STATE (message as pmp_predict_host's).  *report (may be NULL) is the
+ * sum over the windows written.  Every return, errors included, leaves no work queued and the handle usable.  Width or
+ * height below 64 (zero blocks) returns PMP_OK without calling either callback. */
+enum { PMP_OUT_VALUES = 1, PMP_OUT_TEXT = 2 };
+typedef struct pmp_window {
+    int first_frame, frames, n_qps;
+    const int8_t *values[4][2];
+    int64_t n_values[4][2];       /* [qp index][0 luma, 1 chroma] */
+    const char *text[4][2];
+    int64_t text_bytes[4][2];
+    pmp_report report;
+} pmp_window;
+typedef int (*pmp_read_cb)(void *user, int first_frame, int frames, void *y, void *u, void *v);
+typedef int (*pmp_write_cb)(void *user, const pmp_window *w);
+int pmp_predict_stream(pmp_handle *h, int n_qps, const int *wsets, int frames, int width, int height, int sample_bytes,
+                       int window_frames, int outputs, pmp_read_cb read, pmp_write_cb write, void *user,
+                       pmp_report *report);
 
 /* Self-test of the TC conv engine against the SIMT engine on random data (GPU).  Returns 0 and the
  * max-abs error in *max_err, or an error.  flags: bit0 ReLU, bit1 identity residual, bit2 attention product,

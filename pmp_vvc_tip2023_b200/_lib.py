@@ -17,6 +17,26 @@ IN_U8, IN_F32 = 0, 1
 c_void_p, c_int, c_int64, c_char_p = ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_char_p
 _P = ctypes.POINTER
 
+class Report(ctypes.Structure):
+    """struct pmp_report (pmp_predict_host)."""
+    _fields_ = [(k, ctypes.c_longlong) for k in ("blocks", "near_tie_blocks", "near_threshold_blocks",
+                                                 "near_threshold_blocks_tight", "fp16_saturation_events")]
+
+    def as_dict(self):
+        return {k: int(getattr(self, k)) for k, _ in self._fields_}
+
+
+class Window(ctypes.Structure):
+    """struct pmp_window (pmp_predict_stream): one window's results, [qp index][0 luma, 1 chroma]."""
+    _fields_ = [("first_frame", c_int), ("frames", c_int), ("n_qps", c_int),
+                ("values", (c_void_p * 2) * 4), ("n_values", (c_int64 * 2) * 4),
+                ("text", (c_void_p * 2) * 4), ("text_bytes", (c_int64 * 2) * 4), ("report", Report)]
+
+
+OUT_VALUES, OUT_TEXT = 1, 2
+READ_CB = ctypes.CFUNCTYPE(c_int, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p)
+WRITE_CB = ctypes.CFUNCTYPE(c_int, c_void_p, _P(Window))
+
 # name -> (restype, argtypes); kept in one table so tests can check the ABI against the header
 SIGNATURES = {
     "pmp_version": (c_int, []),
@@ -50,6 +70,9 @@ SIGNATURES = {
                                     c_void_p]),
     "pmp_frame_values": (c_int64, [c_int, c_int]),
     "pmp_format_text": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, _P(c_int64), c_void_p]),
+    "pmp_format_texts": (c_int, [c_void_p, c_int, _P(c_void_p), _P(c_int64), _P(c_void_p), c_void_p, c_void_p]),
+    "pmp_predict_stream": (c_int, [c_void_p, c_int, _P(c_int), c_int, c_int, c_int, c_int, c_int, c_int, READ_CB, WRITE_CB,
+                                   c_void_p, _P(Report)]),
     "pmp_cut_blocks": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p,
                                c_void_p]),
     "pmp_run_component": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int, c_int, c_int, c_void_p,
@@ -68,15 +91,6 @@ _lock = threading.Lock()
 
 class PmpError(RuntimeError):
     pass
-
-
-class Report(ctypes.Structure):
-    """struct pmp_report (pmp_predict_host)."""
-    _fields_ = [(k, ctypes.c_longlong) for k in ("blocks", "near_tie_blocks", "near_threshold_blocks",
-                                                 "near_threshold_blocks_tight", "fp16_saturation_events")]
-
-    def as_dict(self):
-        return {k: int(getattr(self, k)) for k, _ in self._fields_}
 
 
 def lib():
@@ -220,3 +234,74 @@ class Handle:
         check(lib().pmp_predict_host(self._h, (c_int * 4)(*wsets), py, pu, pv, y.itemsize, sy, sc, f, wid, hgt, int(chunk),
                                      ptr[0], ptr[1], ctypes.byref(report)))
         return res
+
+    def predict_stream(self, wsets_by_qp, frames, width, height, sample_bytes, read, write, window_frames=0,
+                       outputs=OUT_VALUES | OUT_TEXT, report=None):
+        """pmp_predict_stream.  wsets_by_qp: one (luma Q, luma MSBD, chroma Q, chroma MSBD) row per QP (1 to 4 rows).
+        read(first_frame, frames, y, u, v) fills numpy views of the library's page-locked planes: y [frames, H, W],
+        u/v [frames, H/2, W/2] (None when no QP runs chroma), uint8 or uint16 after sample_bytes.
+        write(w) receives a StreamWindow per window, in frame order; its arrays are views valid only during the call.
+        A non-zero return of a callback aborts the call (PmpError, error -6); an exception raised in a callback aborts
+        it too and is re-raised here, chained to that error.  Returns the Report summed over the windows written."""
+        import numpy as np
+
+        rows = [list(r) for r in wsets_by_qp]
+        nq = len(rows)
+        flat = (c_int * (4 * max(nq, 1)))(*[w for r in rows for w in r])
+        dt = np.uint8 if sample_bytes == 1 else np.uint16
+        raised = []
+
+        def view(ptr, shape, dtype):
+            n = int(np.prod(shape)) * np.dtype(dtype).itemsize
+            if not ptr:
+                return None
+            if n == 0:
+                return np.empty(shape, dtype)
+            return np.frombuffer((ctypes.c_char * n).from_address(ptr), dtype).reshape(shape)
+
+        def on_read(_user, f0, nf, y, u, v):
+            try:
+                r = read(f0, nf, view(y, (nf, height, width), dt), view(u, (nf, height // 2, width // 2), dt),
+                         view(v, (nf, height // 2, width // 2), dt))
+                return int(r or 0)
+            except BaseException as e:          # noqa: B036 -- handed back to the caller below
+                raised.append(e)
+                return 1
+
+        def on_write(_user, wp):
+            try:
+                r = write(StreamWindow(wp.contents, view))
+                return int(r or 0)
+            except BaseException as e:          # noqa: B036
+                raised.append(e)
+                return 1
+
+        report = Report() if report is None else report
+        rc = lib().pmp_predict_stream(self._h, nq, flat, int(frames), int(width), int(height), int(sample_bytes),
+                                      int(window_frames), int(outputs), READ_CB(on_read), WRITE_CB(on_write), None,
+                                      ctypes.byref(report))
+        if raised:
+            try:
+                check(rc)
+            except PmpError:
+                raise raised[0]
+        check(rc)
+        return report
+
+
+class StreamWindow:
+    """One window of pmp_predict_stream: first_frame, frames, n_qps, report (dict) and, keyed by (qp index, component
+    0 luma / 1 chroma), values (int8 [frames * per]) and text (uint8) numpy views of library memory, valid only during
+    the write callback.  Results not computed or not asked for are absent."""
+
+    def __init__(self, w, view):
+        import numpy as np
+        self.first_frame, self.frames, self.n_qps = w.first_frame, w.frames, w.n_qps
+        self.report = w.report.as_dict()
+        self.values, self.text = {}, {}
+        for q in range(w.n_qps):
+            for c in range(2):
+                if w.values[q][c]:
+                    self.values[(q, c)] = view(w.values[q][c], (w.n_values[q][c],), np.int8)
+                if w.text[q][c]:
+                    self.text[(q, c)] = view(w.text[q][c], (w.text_bytes[q][c],), np.uint8)

@@ -6,10 +6,10 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libpmp_b200.so")
 SOURCES = ["api.cu", "nets.cu", "decode.cu", "conv_simt.cu", "conv_tc.cu"]
-# host-level entry points (pmp_weights_load, pmp_predict_host) on top of the core; their pmp_destroy releases the host
-# staging and then runs csrc/api.cu's, which is compiled under another name for that
+# host-level entry points (pmp_weights_load, pmp_predict_host, pmp_predict_stream, pmp_format_texts) on top of the core;
+# their pmp_destroy releases the host staging and then runs csrc/api.cu's, which is compiled under another name for that
 HOST = os.path.join(HERE, "host")
-HOST_SOURCES = ["host_api.cu"]
+HOST_SOURCES = ["host_api.cu", "text_batch.cu"]
 SOURCE_DEFINES = {"api.cu": ["-Dpmp_destroy=pmp_destroy_core"]}
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--use_fast_math=false"]

@@ -2,6 +2,7 @@
 //
 //   pmp_predict --input SEQ.yuv --width W --height H --frames N [--bitDepth 8|10] [--ssRatio S] [--qps 22,27,32,37]
 //               --modelDir DIR --outDir DIR [--binaryOut] [--device D] [--tcDtype fp16|bf16] [--chunk C] [--timing]
+//               [--stream]
 //
 // The weights are the exported .pmpw files (python -m pmp_vvc_tip2023_b200.export_weights): <comp>_Q_<qp>.pmpw and
 // <comp>_BD_<qp>.pmpw in --modelDir.  Frames are read as Inference_QBD.import_yuv420 reads them (every S-th frame, by
@@ -11,6 +12,12 @@
 // tools/vtm_reader/pmp_partition_reader.h).  Without --binaryOut an existing .bin is deleted, so that the VTM-side reader
 // cannot pick up a stale one.  Nothing is written when the fp16 range guard fired (exit status 1: rerun with
 // --tcDtype bf16).
+//
+// --stream makes one pmp_predict_stream call for all QPs instead: frames are read window by window straight into the
+// library's page-locked planes, the GPU formats the text, and each window's text (and .bin payload) is appended to
+// <stem>.txt.part (.bin.part) while the next window computes; the .part files are renamed once the call succeeds and
+// deleted otherwise, so existing files are left as they were.  Host memory is bounded by the window (--chunk blocks,
+// default 4800), not by the sequence.  The files are the same as without --stream.
 #include "pmp_b200.h"
 
 #include <chrono>
@@ -27,7 +34,7 @@ struct Args {
     std::string input, model_dir, out_dir;
     int width = 0, height = 0, frames = 0, bit_depth = 8, ss_ratio = 1, device = 0, chunk = 0;
     std::vector<int> qps{22, 27, 32, 37};
-    bool binary_out = false, bf16 = false, timing = false;
+    bool binary_out = false, bf16 = false, timing = false, stream = false;
 };
 
 int usage(const char *msg)
@@ -35,7 +42,7 @@ int usage(const char *msg)
     std::fprintf(stderr,
                  "pmp_predict: %s\nusage: pmp_predict --input SEQ.yuv --width W --height H --frames N [--bitDepth 8|10] "
                  "[--ssRatio S] [--qps 22,27,32,37] --modelDir DIR --outDir DIR [--binaryOut] [--device D] "
-                 "[--tcDtype fp16|bf16] [--chunk C] [--timing]\n",
+                 "[--tcDtype fp16|bf16] [--chunk C] [--timing] [--stream]\n",
                  msg);
     return 2;
 }
@@ -46,6 +53,7 @@ bool parse(int argc, char **argv, Args &a, std::string &err)
         const std::string k = argv[i];
         if (k == "--binaryOut") { a.binary_out = true; continue; }
         if (k == "--timing") { a.timing = true; continue; }
+        if (k == "--stream") { a.stream = true; continue; }
         if (i + 1 >= argc) { err = "missing value for " + k; return false; }
         const std::string v = argv[++i];
         if (k == "--input") a.input = v;
@@ -132,6 +140,142 @@ int fail(const char *what)
     return 1;
 }
 
+void print_report(const pmp_report &tot)
+{
+    const double near_tol = 1e-2;      // the library's default (pmp_set_near_tol)
+    std::printf("Decode report: %lld block-QPs, %lld float32 near-tie argmins, %lld with a map value within %g of a decision "
+                "threshold (%lld within %g), %lld fp16 saturation events\n",
+                tot.blocks, tot.near_tie_blocks, tot.near_threshold_blocks, near_tol, tot.near_threshold_blocks_tight,
+                0.01 * near_tol, tot.fp16_saturation_events);
+}
+
+int saturated_exit(long long events)
+{
+    std::fprintf(stderr, "pmp_predict: activations left the fp16 range (%lld events): results are clamped; rerun with "
+                         "--tcDtype bf16\n", events);
+    return 1;
+}
+
+std::string stem_of(const Args &a, const std::string &base, int qp, int c)
+{
+    static const char *const comps[2] = {"Luma", "Chroma"};
+    return a.out_dir + "/" + base + "_" + comps[c] + "_QP" + std::to_string(qp) + "_PartitionMat";
+}
+
+// ---- --stream ------------------------------------------------------------------------------------------------------
+struct Stream {
+    const Args *a;
+    FILE *in = nullptr;
+    size_t ysz = 0, csz = 0;
+    int sb = 1;
+    std::vector<FILE *> txt, bin;      // [2 * qp index + component]
+    std::string io_error;
+};
+
+// Inference_QBD.import_yuv420's frames [f0, f0 + nf) of the subsampled sequence, into the library's planes
+int stream_read(void *user, int f0, int nf, void *y, void *u, void *v)
+{
+    Stream &st = *static_cast<Stream *>(user);
+    const Args &a = *st.a;
+    for (int k = 0; k < nf; k++) {
+        const long long off = (long long)(f0 + k) * a.ss_ratio * (long long)(st.ysz + 2 * st.csz);
+        bool ok = fseeko(st.in, (off_t)off, SEEK_SET) == 0 && std::fread((char *)y + k * st.ysz, 1, st.ysz, st.in) == st.ysz;
+        if (ok && u)
+            ok = std::fread((char *)u + k * st.csz, 1, st.csz, st.in) == st.csz &&
+                 std::fread((char *)v + k * st.csz, 1, st.csz, st.in) == st.csz;
+        if (!ok) {
+            st.io_error = a.input + " holds fewer than " + std::to_string(a.frames) + " frames of " + std::to_string(a.width) +
+                          "x" + std::to_string(a.height);
+            return 1;
+        }
+    }
+    return 0;
+}
+
+int stream_write(void *user, const pmp_window *w)
+{
+    Stream &st = *static_cast<Stream *>(user);
+    for (int q = 0; q < w->n_qps; q++)
+        for (int c = 0; c < 2; c++) {
+            const size_t i = 2 * q + c, nt = (size_t)w->text_bytes[q][c], nv = (size_t)w->n_values[q][c];
+            if (std::fwrite(w->text[q][c], 1, nt, st.txt[i]) != nt || (st.bin[i] && std::fwrite(w->values[q][c], 1, nv, st.bin[i]) != nv)) {
+                st.io_error = "write error";
+                return 1;
+            }
+        }
+    return 0;
+}
+
+int run_stream(const Args &a, pmp_handle *h, const std::vector<int> &wsets, const std::string &base)
+{
+    Stream st;
+    st.a = &a;
+    st.sb = a.bit_depth == 10 ? 2 : 1;
+    st.ysz = (size_t)a.width * a.height * st.sb;
+    st.csz = st.ysz / 4;
+    const int nf = (a.frames + a.ss_ratio - 1) / a.ss_ratio, bh = a.height / 64, bw = a.width / 64, bpf = bh * bw;
+    st.in = std::fopen(a.input.c_str(), "rb");
+    if (!st.in) { std::fprintf(stderr, "pmp_predict: cannot open %s\n", a.input.c_str()); return 1; }
+    mkdir(a.out_dir.c_str(), 0777);      // an existing directory is fine; a failure shows when the files are opened
+    std::vector<std::string> parts;
+    bool ok = true;
+    for (size_t q = 0; q < a.qps.size() && ok; q++)
+        for (int c = 0; c < 2 && ok; c++) {
+            const std::string stem = stem_of(a, base, a.qps[q], c);
+            parts.push_back(stem + ".txt.part");
+            FILE *t = std::fopen(parts.back().c_str(), "wb");
+            FILE *b = nullptr;
+            if (t && a.binary_out) {
+                parts.push_back(stem + ".bin.part");
+                b = std::fopen(parts.back().c_str(), "wb");
+                int32_t head32[8] = {0, 0, nf, 16 * bh, 16 * bw, 0, 0, 0};      // PMPPART1, frames, R, C, reserved
+                std::memcpy(head32, "PMPPART1", 8);
+                ok = b && std::fwrite(head32, 1, sizeof head32, b) == sizeof head32;
+            }
+            ok = ok && t;
+            st.txt.push_back(t);
+            st.bin.push_back(b);
+            if (!ok) std::fprintf(stderr, "pmp_predict: cannot write %s\n", parts.back().c_str());
+        }
+    int rc = PMP_OK;
+    pmp_report tot = {0, 0, 0, 0, 0};
+    if (ok) {
+        const auto t0 = std::chrono::steady_clock::now();
+        const int window = a.chunk > 0 && bpf > 0 ? std::max(1, a.chunk / bpf) : 0;
+        rc = pmp_predict_stream(h, (int)a.qps.size(), wsets.data(), nf, a.width, a.height, st.sb, window,
+                                PMP_OUT_TEXT | (a.binary_out ? PMP_OUT_VALUES : 0), stream_read, stream_write, &st, &tot);
+        const double ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+        const int wf = window > 0 ? window : std::max(1, bpf > 0 ? 4800 / bpf : 1);
+        if (a.timing) std::printf("pmp_predict_stream %.3f ms (%d frames, %d windows)\n", ms, nf, bpf > 0 ? (nf + wf - 1) / wf : 0);
+    }
+    std::fclose(st.in);
+    for (size_t i = 0; i < st.txt.size(); i++) {
+        if (st.txt[i] && std::fclose(st.txt[i]) != 0) st.io_error = "write error";
+        if (st.bin[i] && std::fclose(st.bin[i]) != 0) st.io_error = "write error";
+    }
+    ok = ok && rc == PMP_OK && st.io_error.empty();
+    if (ok) print_report(tot);
+    for (size_t q = 0; q < a.qps.size() && ok; q++)
+        for (int c = 0; c < 2 && ok; c++) {
+            const std::string stem = stem_of(a, base, a.qps[q], c);
+            ok = std::rename((stem + ".txt.part").c_str(), (stem + ".txt").c_str()) == 0;
+            if (ok && a.binary_out) ok = std::rename((stem + ".bin.part").c_str(), (stem + ".bin").c_str()) == 0;
+            else if (ok) std::remove((stem + ".bin").c_str());
+            if (ok) std::printf("Save: %s.txt\n", stem.c_str());
+            else std::fprintf(stderr, "pmp_predict: cannot rename %s.*.part\n", stem.c_str());
+        }
+    if (ok) return 0;
+    for (const std::string &p : parts) std::remove(p.c_str());
+    if (rc == PMP_ERR_STATE && tot.fp16_saturation_events) {
+        print_report(tot);
+        std::fprintf(stderr, "pmp_predict: %s\n", pmp_last_error());
+        return saturated_exit(tot.fp16_saturation_events);
+    }
+    if (!st.io_error.empty()) std::fprintf(stderr, "pmp_predict: %s\n", st.io_error.c_str());
+    if (rc != PMP_OK) return fail("pmp_predict_stream");
+    return 1;
+}
+
 }  // namespace
 
 int main(int argc, char **argv)
@@ -157,6 +301,14 @@ int main(int argc, char **argv)
                     return 1;
                 }
             }
+
+    std::string base = a.input.substr(a.input.find_last_of('/') + 1);
+    if (base.size() > 4 && base.compare(base.size() - 4, 4, ".yuv") == 0) base.resize(base.size() - 4);
+    if (a.stream) {
+        rc = run_stream(a, h, wsets, base);
+        pmp_destroy(h);
+        return rc;
+    }
 
     const int sb = a.bit_depth == 10 ? 2 : 1;
     std::vector<char> yuv;
@@ -190,23 +342,13 @@ int main(int argc, char **argv)
         tot.fp16_saturation_events += r.fp16_saturation_events;
     }
     pmp_destroy(h);
-    const double near_tol = 1e-2;      // the library's default (pmp_set_near_tol)
-    std::printf("Decode report: %lld block-QPs, %lld float32 near-tie argmins, %lld with a map value within %g of a decision "
-                "threshold (%lld within %g), %lld fp16 saturation events\n",
-                tot.blocks, tot.near_tie_blocks, tot.near_threshold_blocks, near_tol, tot.near_threshold_blocks_tight,
-                0.01 * near_tol, tot.fp16_saturation_events);
-    if (saturated) {
-        std::fprintf(stderr, "pmp_predict: activations left the fp16 range (%lld events): results are clamped; rerun with "
-                             "--tcDtype bf16\n", tot.fp16_saturation_events);
-        return 1;
-    }
+    print_report(tot);
+    if (saturated) return saturated_exit(tot.fp16_saturation_events);
 
     mkdir(a.out_dir.c_str(), 0777);      // an existing directory is fine; a failure shows when the files are written
-    std::string base = a.input.substr(a.input.find_last_of('/') + 1);
-    if (base.size() > 4 && base.compare(base.size() - 4, 4, ".yuv") == 0) base.resize(base.size() - 4);
     for (size_t q = 0; q < a.qps.size(); q++)
         for (int c = 0; c < 2; c++) {
-            const std::string stem = a.out_dir + "/" + base + "_" + comps[c] + "_QP" + std::to_string(a.qps[q]) + "_PartitionMat";
+            const std::string stem = stem_of(a, base, a.qps[q], c);
             std::printf("Save: %s.txt\n", stem.c_str());
             if (!write_text(stem + ".txt", out[2 * q + c])) return 1;
             if (a.binary_out) {
