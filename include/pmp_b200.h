@@ -35,7 +35,7 @@ enum pmp_status {
     PMP_ERR_NO_DEVICE = -3,
     PMP_ERR_STATE = -4,    /* unknown weight set, wrong net kind ... */
     PMP_ERR_UNSUPPORTED = -5,
-    PMP_ERR_ABORTED = -6   /* a callback of pmp_predict_stream returned non-zero (message names it and its value) */
+    PMP_ERR_ABORTED = -6   /* a callback of pmp_predict_stream(_multi) returned non-zero (message names it and its value) */
 };
 
 /* Net kinds: Model_QBD.py:59 Luma_Q_Net, :100 Luma_MSBD_Net, :157 Chroma_Q_Net, :198 Chroma_MSBD_Net */
@@ -219,6 +219,26 @@ typedef int (*pmp_write_cb)(void *user, const pmp_window *w);
 int pmp_predict_stream(pmp_handle *h, int n_qps, const int *wsets, int frames, int width, int height, int sample_bytes,
                        int window_frames, int outputs, pmp_read_cb read, pmp_write_cb write, void *user,
                        pmp_report *report);
+
+/* pmp_predict_stream_multi: pmp_predict_stream over several handles at once, on one or several devices (the same
+ * sequence and files, several GPUs busy).  handles: n_handles (1..16) distinct non-NULL handles; they may share a device,
+ * each keeps its own streams and staging.  wsets: [n_handles][n_qps][4]; row [i][q] names handles[i]'s weight sets for
+ * QP q (ids are per handle).
+ * Before any callback the call checks that every handle computes what handles[0] computes: the same skip pattern, net
+ * kinds and weights (an FNV-1a-64 fingerprint of each weight set's fp32 parameters, taken once per handle and weight set),
+ * the same engine and tc_dtype (pmp_set_engine) and the same near_tol (pmp_set_near_tol).  Otherwise it returns
+ * PMP_ERR_ARG, calls no callback, and the message names the handle index and the first item that differs.
+ * Window k runs on handles[k % n_handles]; each handle keeps its two window slots busy, so up to 2 * n_handles windows
+ * are in flight, and the host blocks only on the download of the oldest window not yet written.  window_frames <= 0:
+ * max(1, min(4800 / blocks per frame, ceil(frames / n_handles))), so that a short sequence still reaches every handle.
+ * The callbacks run on the calling thread, with the calling thread's current device made current before each of them
+ * (the call switches devices in between and restores the device on return): read in ascending, contiguous frame order,
+ * each frame once; write once per window, in frame order.  All other arguments, the callbacks' contract, the errors,
+ * the saturation stop and *report are those of pmp_predict_stream: every return leaves no work queued on any handle and
+ * every handle usable.  The values and text are byte-identical to pmp_predict_stream on handles[0]. */
+int pmp_predict_stream_multi(pmp_handle *const *handles, int n_handles, int n_qps, const int *wsets, int frames,
+                             int width, int height, int sample_bytes, int window_frames, int outputs, pmp_read_cb read,
+                             pmp_write_cb write, void *user, pmp_report *report);
 
 /* Self-test of the TC conv engine against the SIMT engine on random data (GPU).  Returns 0 and the
  * max-abs error in *max_err, or an error.  flags: bit0 ReLU, bit1 identity residual, bit2 attention product,

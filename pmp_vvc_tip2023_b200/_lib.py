@@ -73,6 +73,8 @@ SIGNATURES = {
     "pmp_format_texts": (c_int, [c_void_p, c_int, _P(c_void_p), _P(c_int64), _P(c_void_p), c_void_p, c_void_p]),
     "pmp_predict_stream": (c_int, [c_void_p, c_int, _P(c_int), c_int, c_int, c_int, c_int, c_int, c_int, READ_CB, WRITE_CB,
                                    c_void_p, _P(Report)]),
+    "pmp_predict_stream_multi": (c_int, [_P(c_void_p), c_int, c_int, _P(c_int), c_int, c_int, c_int, c_int, c_int, c_int,
+                                         READ_CB, WRITE_CB, c_void_p, _P(Report)]),
     "pmp_cut_blocks": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p,
                                c_void_p]),
     "pmp_run_component": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int, c_int, c_int, c_void_p,
@@ -243,50 +245,73 @@ class Handle:
         write(w) receives a StreamWindow per window, in frame order; its arrays are views valid only during the call.
         A non-zero return of a callback aborts the call (PmpError, error -6); an exception raised in a callback aborts
         it too and is re-raised here, chained to that error.  Returns the Report summed over the windows written."""
-        import numpy as np
-
         rows = [list(r) for r in wsets_by_qp]
-        nq = len(rows)
-        flat = (c_int * (4 * max(nq, 1)))(*[w for r in rows for w in r])
-        dt = np.uint8 if sample_bytes == 1 else np.uint16
-        raised = []
+        flat = (c_int * (4 * max(len(rows), 1)))(*[w for r in rows for w in r])
+        return _stream_call(lambda rd, wr, rep: lib().pmp_predict_stream(
+            self._h, len(rows), flat, int(frames), int(width), int(height), int(sample_bytes), int(window_frames),
+            int(outputs), rd, wr, None, rep), width, height, sample_bytes, read, write, report)
 
-        def view(ptr, shape, dtype):
-            n = int(np.prod(shape)) * np.dtype(dtype).itemsize
-            if not ptr:
-                return None
-            if n == 0:
-                return np.empty(shape, dtype)
-            return np.frombuffer((ctypes.c_char * n).from_address(ptr), dtype).reshape(shape)
 
-        def on_read(_user, f0, nf, y, u, v):
-            try:
-                r = read(f0, nf, view(y, (nf, height, width), dt), view(u, (nf, height // 2, width // 2), dt),
-                         view(v, (nf, height // 2, width // 2), dt))
-                return int(r or 0)
-            except BaseException as e:          # noqa: B036 -- handed back to the caller below
-                raised.append(e)
-                return 1
+def predict_stream_multi(handles, wsets_by_handle, frames, width, height, sample_bytes, read, write, window_frames=0,
+                         outputs=OUT_VALUES | OUT_TEXT, report=None):
+    """pmp_predict_stream_multi: Handle.predict_stream over several handles (1 to 16, on one or several devices), window
+    k on handles[k % len(handles)].  wsets_by_handle[i]: handles[i]'s rows, one (luma Q, luma MSBD, chroma Q,
+    chroma MSBD) per QP, the same QPs and weights on every handle.  The callbacks, errors and result are those of
+    Handle.predict_stream; the calling thread's current device is current inside the callbacks and after the call."""
+    nh = len(handles)
+    rows = [[list(r) for r in by_qp] for by_qp in wsets_by_handle]
+    nq = len(rows[0]) if rows else 0
+    if len(rows) != nh or any(len(r) != nq for r in rows):
+        raise ValueError("wsets_by_handle needs one list of %d QP rows per handle" % nq)
+    flat = (c_int * (4 * max(nh * nq, 1)))(*[w for by_qp in rows for r in by_qp for w in r])
+    hs = (c_void_p * max(nh, 1))(*[h.ptr if isinstance(h, Handle) else h for h in handles])
+    return _stream_call(lambda rd, wr, rep: lib().pmp_predict_stream_multi(
+        hs, nh, nq, flat, int(frames), int(width), int(height), int(sample_bytes), int(window_frames), int(outputs), rd,
+        wr, None, rep), width, height, sample_bytes, read, write, report)
 
-        def on_write(_user, wp):
-            try:
-                r = write(StreamWindow(wp.contents, view))
-                return int(r or 0)
-            except BaseException as e:          # noqa: B036
-                raised.append(e)
-                return 1
 
-        report = Report() if report is None else report
-        rc = lib().pmp_predict_stream(self._h, nq, flat, int(frames), int(width), int(height), int(sample_bytes),
-                                      int(window_frames), int(outputs), READ_CB(on_read), WRITE_CB(on_write), None,
-                                      ctypes.byref(report))
-        if raised:
-            try:
-                check(rc)
-            except PmpError:
-                raise raised[0]
-        check(rc)
-        return report
+def _stream_call(call, width, height, sample_bytes, read, write, report):
+    """Runs call(read_cb, write_cb, report_ptr) -> status with the Python callbacks of predict_stream wrapped: numpy views
+    of the planes and StreamWindows in, a callback's exception re-raised here chained to the -6 it caused."""
+    import numpy as np
+
+    dt = np.uint8 if sample_bytes == 1 else np.uint16
+    raised = []
+
+    def view(ptr, shape, dtype):
+        n = int(np.prod(shape)) * np.dtype(dtype).itemsize
+        if not ptr:
+            return None
+        if n == 0:
+            return np.empty(shape, dtype)
+        return np.frombuffer((ctypes.c_char * n).from_address(ptr), dtype).reshape(shape)
+
+    def on_read(_user, f0, nf, y, u, v):
+        try:
+            r = read(f0, nf, view(y, (nf, height, width), dt), view(u, (nf, height // 2, width // 2), dt),
+                     view(v, (nf, height // 2, width // 2), dt))
+            return int(r or 0)
+        except BaseException as e:          # noqa: B036 -- handed back to the caller below
+            raised.append(e)
+            return 1
+
+    def on_write(_user, wp):
+        try:
+            r = write(StreamWindow(wp.contents, view))
+            return int(r or 0)
+        except BaseException as e:          # noqa: B036
+            raised.append(e)
+            return 1
+
+    report = Report() if report is None else report
+    rc = call(READ_CB(on_read), WRITE_CB(on_write), ctypes.byref(report))
+    if raised:
+        try:
+            check(rc)
+        except PmpError:
+            raise raised[0]
+    check(rc)
+    return report
 
 
 class StreamWindow:

@@ -1,7 +1,7 @@
 // Host-level entry points of libpmp_b200 for callers without Python or CUDA of their own (include/pmp_b200.h):
 // pmp_weights_load (exported .pmpw weight files), pmp_predict_host (host planes in, host PartitionMat vectors out),
-// pmp_predict_stream (frames in through a callback, every QP's vectors and text out window by window) and
-// pmp_format_texts (text_batch.cu), plus pmp_destroy, which releases this layer's staging before the core handle
+// pmp_predict_stream (frames in through a callback, every QP's vectors and text out window by window),
+// pmp_predict_stream_multi (the same over several handles, windows in rotation) and pmp_format_texts (text_batch.cu), plus pmp_destroy, which releases this layer's staging before the core handle
 // teardown in csrc/api.cu.
 //
 // This layer only calls the core's entry points and internal functions; it lives outside csrc/ because bench.py ties
@@ -11,6 +11,7 @@
 #include "host.cuh"
 
 #include <algorithm>
+#include <climits>
 #include <cstdio>
 #include <cstring>
 #include <functional>
@@ -79,9 +80,8 @@ std::vector<Param> net_params(int net)
     return v;
 }
 
-uint64_t fnv1a64(const unsigned char *p, size_t n)
+uint64_t fnv1a64(const unsigned char *p, size_t n, uint64_t x = 0xcbf29ce484222325ull)
 {
-    uint64_t x = 0xcbf29ce484222325ull;
     for (size_t i = 0; i < n; i++) x = (x ^ p[i]) * 0x100000001b3ull;
     return x;
 }
@@ -159,12 +159,13 @@ int weights_load(Handle *h, const char *path, int *net_out, int *wset)
     return rc;
 }
 
-// ---- the window pipeline of pmp_predict_host and pmp_predict_stream ----------------------------------------------
+// ---- the window pipeline of pmp_predict_host, pmp_predict_stream and pmp_predict_stream_multi ---------------------
 // Per handle: a compute and a copy stream, their events, and per window slot (double-buffered) pinned + device buffers
 // for the input planes and for the results (values, decode flags and, when asked for, text of every (QP, component)
 // pair, the text byte counts and a snapshot of the saturation counter).  Created on first use, grown to the largest
 // window, released by pmp_destroy.
 constexpr int RESULTS_MAX = 8;      // 4 QPs x 2 components
+constexpr int STREAM_HANDLES_MAX = 16;     // handles of one pmp_predict_stream_multi call
 
 struct HostStage {
     cudaStream_t compute = nullptr, copy = nullptr;
@@ -286,10 +287,53 @@ int saturation_error(long long events)
     return PMP_ERR_STATE;
 }
 
+// ---- weight fingerprints (pmp_predict_stream_multi's check that every handle holds the same weights) ----------------
+// FNV-1a-64 over a weight set's exact fp32 parameters as the SIMT engine holds them: every conv's name, shape, packed
+// weight image and bias, in the set's name order.  Copied to the host once per (handle, weight set): ids are never
+// reused within a handle (next_wset++), and pmp_destroy drops the handle's entries.
+std::mutex g_fp_mu;
+std::map<std::pair<const Handle *, int>, uint64_t> g_fingerprint;
+
+int wset_fingerprint(Handle *h, int id, uint64_t *out)
+{
+    {
+        std::lock_guard<std::mutex> lock(g_fp_mu);
+        auto it = g_fingerprint.find({h, id});
+        if (it != g_fingerprint.end()) { *out = it->second; return PMP_OK; }
+    }
+    PMP_CUDA(cudaSetDevice(h->device));
+    uint64_t x = fnv1a64(nullptr, 0);
+    std::vector<float> buf;
+    for (const auto &kv : h->wsets.at(id).convs) {      // the caller checked that the set exists
+        const ConvW &cw = kv.second;
+        const int dims[4] = {cw.cout, cw.cin, cw.kh, cw.kw};
+        x = fnv1a64((const unsigned char *)kv.first.data(), kv.first.size(), x);
+        x = fnv1a64((const unsigned char *)dims, sizeof dims, x);
+        const float *part[2] = {cw.w_simt, cw.bias};
+        const size_t n[2] = {cw.w_simt ? (size_t)cw.cin * cw.kh * cw.kw * ((cw.cout + 3) & ~3) : 0,   // nets.cu's layout
+                             cw.bias ? (size_t)cw.cout : 0};
+        for (int p = 0; p < 2; p++) {
+            buf.resize(n[p]);
+            if (n[p]) PMP_CUDA(cudaMemcpy(buf.data(), part[p], n[p] * sizeof(float), cudaMemcpyDeviceToHost));
+            x = fnv1a64((const unsigned char *)buf.data(), n[p] * sizeof(float), x);
+        }
+    }
+    std::lock_guard<std::mutex> lock(g_fp_mu);
+    g_fingerprint[{h, id}] = x;
+    *out = x;
+    return PMP_OK;
+}
+
+void release_fingerprints(const Handle *h)
+{
+    std::lock_guard<std::mutex> lock(g_fp_mu);
+    g_fingerprint.erase(g_fingerprint.lower_bound({h, INT_MIN}), g_fingerprint.upper_bound({h, INT_MAX}));
+}
+
 // One call's work: the (QP, component) results over `frames` frames, in windows of `wf` whole frames.  The entry point
 // supplies the host ends of a window: fill() provides its input planes, write() takes its results.
 struct WindowJob {
-    int n_qps = 0, wsets[4][4] = {}, frames = 0, width = 0, height = 0, sample_bytes = 1, wf = 1, chunk = 4800;
+    int n_qps = 0, frames = 0, width = 0, height = 0, sample_bytes = 1, wf = 1, chunk = 4800;
     bool on[4][2] = {};
     bool values = true, text = false;       // download the values; format and download the text
     bool stop_on_saturation = false;        // stop after the first window with saturation events, or finish them all
@@ -302,10 +346,23 @@ struct WindowJob {
     std::function<int(const pmp_window &w)> write;      // returns a pmp_status
 };
 
-// Runs `job`: window k+1 is filled and uploaded and window k-1 downloaded and written while window k computes; each
-// window is cut into blocks once for all its results.  The host waits only on events of finished windows.  *total
-// receives the sum of the reports of the windows written.  Every return leaves no work queued.
-int run_windows(pmp_handle *h, const WindowJob &job, pmp_report *total)
+// One handle's part of a call: windows k with k % lanes == its index, on its own streams and staging.
+struct Lane {
+    pmp_handle *h = nullptr;
+    const int *wsets = nullptr;     // [n_qps][4]: this handle's weight-set ids
+    HostStage *st = nullptr;        // set by run_windows
+    unsigned int sat_prev = 0;      // the handle's saturation counter after its previous window
+};
+
+// Runs `job` over the lanes in rotation: window k runs on lanes[k % n].  Iteration k computes window k, fills and
+// uploads window k + n, downloads window k and writes window k - n, so each lane keeps both its window slots busy while
+// the host reads and writes in frame order; with one lane, window k+1 is filled and uploaded and window k-1 written
+// while window k computes.  Each lane's first window is computed as soon as it is uploaded, so that no device waits for
+// the other lanes' first reads.  Each window is cut into blocks once for all its results.  The host waits only on
+// events of finished windows.  The device of a lane is made current before each of its CUDA calls; fill() and write()
+// may switch devices.  *total receives the sum of the reports of the windows written.  Every return leaves no work
+// queued on any lane.
+int run_windows(std::vector<Lane> &lanes, const WindowJob &job, pmp_report *total)
 {
     memset(total, 0, sizeof(*total));
     const int bh = job.height / 64, bw = job.width / 64, bpf = bh * bw, wf = job.wf, frames = job.frames;
@@ -341,34 +398,44 @@ int run_windows(pmp_handle *h, const WindowJob &job, pmp_report *total)
     }
     const size_t off_nbytes = off, off_sat = off + 8 * RESULTS_MAX;
     const size_t blk_bytes[2] = {(size_t)68 * 68, (size_t)3 * 34 * 34};
-    HostStage &st = stage_of(h);
-    int rc = ensure_stage(st, (size_t)wf * in_frame, off_sat + 256,
-                          (size_t)nmax * ((comp_on[0] ? blk_bytes[0] : 0) + (comp_on[1] ? blk_bytes[1] : 0)));
-    if (rc) return rc;
-    // The status word and the text status words exist before the loop (allocating them synchronises the device).  The
-    // arena and scratch grow inside the first window's pmp_run_component when a handle first sees this window size; that
-    // synchronises the device once and leaves everything queued intact.
-    if ((rc = ensure_status(h))) return rc;
-    if (job.text && (rc = reserve_text_status(h, nres, (long long)wf * per))) return rc;
-    PMP_CUDA(cudaDeviceSynchronize());
-    unsigned int sat_prev = 0;
-    PMP_CUDA(cudaMemcpy(&sat_prev, h->d_status, sizeof(sat_prev), cudaMemcpyDeviceToHost));
-
     const int nwin = (frames + wf - 1) / wf;
+    if ((int)lanes.size() > nwin) lanes.resize(nwin);       // lanes without a window stay untouched
+    const int n = (int)lanes.size();
+    int rc = PMP_OK;
+    for (Lane &ln : lanes) {
+        pmp_handle *h = ln.h;
+        PMP_CUDA(cudaSetDevice(h->device));
+        ln.st = &stage_of(h);
+        rc = ensure_stage(*ln.st, (size_t)wf * in_frame, off_sat + 256,
+                          (size_t)nmax * ((comp_on[0] ? blk_bytes[0] : 0) + (comp_on[1] ? blk_bytes[1] : 0)));
+        if (rc) return rc;
+        // The status word and the text status words exist before the loop (allocating them synchronises the device).
+        // The arena and scratch grow inside the first window's pmp_run_component when a handle first sees this window
+        // size; that synchronises the device once and leaves everything queued intact.
+        if ((rc = ensure_status(h))) return rc;
+        if (job.text && (rc = reserve_text_status(h, nres, (long long)wf * per))) return rc;
+        PMP_CUDA(cudaDeviceSynchronize());
+        PMP_CUDA(cudaMemcpy(&ln.sat_prev, h->d_status, sizeof(ln.sat_prev), cudaMemcpyDeviceToHost));
+    }
+
     auto win_frames = [&](int k) { return std::min(wf, frames - k * wf); };
     auto direct = [&](int f0, int i) -> int8_t * { return job.direct_out ? job.direct_out(f0, res_q[i], res_c[i]) : nullptr; };
 
     auto upload = [&](int k) -> int {
-        const int s = k & 1, f0 = k * wf, nf = win_frames(k);
-        if (k >= 2) {
+        Lane &ln = lanes[k % n];
+        HostStage &st = *ln.st;
+        const int j = k / n, s = j & 1, f0 = k * wf, nf = win_frames(k);      // j: the lane's own window count
+        PMP_CUDA(cudaSetDevice(ln.h->device));
+        if (j >= 2) {
             if (!job.direct_in) PMP_CUDA(cudaEventSynchronize(st.uploaded[s]));     // pin_in[s] free again
-            PMP_CUDA(cudaStreamWaitEvent(st.copy, st.cut[s], 0));                   // dev_in[s] read by window k-2's cut
+            PMP_CUDA(cudaStreamWaitEvent(st.copy, st.cut[s], 0));                   // dev_in[s] read by the cut of j-2
         }
         char *pin[3] = {nullptr, nullptr, nullptr};
         const char *src[3] = {nullptr, nullptr, nullptr};
         for (int p = 0; p < nplanes; p++) src[p] = pin[p] = st.pin_in[s] + in_off(p, nf);
         int r = job.fill(f0, nf, pin, src);
         if (r) return r;
+        PMP_CUDA(cudaSetDevice(ln.h->device));
         for (int p = 0; p < nplanes; p++)
             PMP_CUDA(cudaMemcpyAsync(st.dev_in[s] + in_off(p, nf), src[p], (size_t)nf * rows[p] * prow[p],
                                      cudaMemcpyHostToDevice, st.copy));
@@ -376,9 +443,13 @@ int run_windows(pmp_handle *h, const WindowJob &job, pmp_report *total)
         return PMP_OK;
     };
     auto compute = [&](int k) -> int {
-        const int s = k & 1, nf = win_frames(k);
+        Lane &ln = lanes[k % n];
+        HostStage &st = *ln.st;
+        pmp_handle *h = ln.h;
+        const int j = k / n, s = j & 1, nf = win_frames(k);
+        PMP_CUDA(cudaSetDevice(h->device));
         PMP_CUDA(cudaStreamWaitEvent(st.compute, st.uploaded[s], 0));
-        if (k >= 2) PMP_CUDA(cudaStreamWaitEvent(st.compute, st.downloaded[s], 0));   // dev_out[s] read by window k-2
+        if (j >= 2) PMP_CUDA(cudaStreamWaitEvent(st.compute, st.downloaded[s], 0));   // dev_out[s] read by j-2
         const char *d = st.dev_in[s];
         char *o = st.dev_out[s];
         uint8_t *blk[2] = {comp_on[0] ? st.dev_blocks : nullptr,
@@ -388,7 +459,7 @@ int run_windows(pmp_handle *h, const WindowJob &job, pmp_report *total)
         if (r) return r;
         PMP_CUDA(cudaEventRecord(st.cut[s], st.compute));
         for (int i = 0; i < nres; i++) {
-            const int *ws = job.wsets[res_q[i]], c = res_c[i];
+            const int *ws = ln.wsets + 4 * res_q[i], c = res_c[i];
             r = pmp_run_component(h, ws[2 * c], ws[2 * c + 1], c == 0, blk[c], nf, bh, bw, job.chunk,
                                   (int8_t *)(o + off_vals[i]), nullptr, nullptr, nullptr, (uint32_t *)(o + off_flags[i]),
                                   st.compute);
@@ -397,23 +468,26 @@ int run_windows(pmp_handle *h, const WindowJob &job, pmp_report *total)
         }
         if (job.text) {
             const int8_t *vals[RESULTS_MAX];
-            int64_t n[RESULTS_MAX];
+            int64_t nv[RESULTS_MAX];
             char *txt[RESULTS_MAX];
             for (int i = 0; i < nres; i++) {
                 vals[i] = (const int8_t *)(o + off_vals[i]);
-                n[i] = (int64_t)nf * per;
+                nv[i] = (int64_t)nf * per;
                 txt[i] = o + off_text[i];
             }
-            if ((r = format_texts(h, nres, vals, n, txt, (int64_t *)(o + off_nbytes), st.compute))) return r;
+            if ((r = format_texts(h, nres, vals, nv, txt, (int64_t *)(o + off_nbytes), st.compute))) return r;
         }
         PMP_CUDA(cudaMemcpyAsync(o + off_sat, h->d_status, sizeof(unsigned int), cudaMemcpyDeviceToDevice, st.compute));
         PMP_CUDA(cudaEventRecord(st.finished[s], st.compute));
         return PMP_OK;
     };
     auto download = [&](int k) -> int {        // a result's values leave while the next result's kernels run
-        const int s = k & 1, f0 = k * wf, nf = win_frames(k);
+        Lane &ln = lanes[k % n];
+        HostStage &st = *ln.st;
+        const int s = (k / n) & 1, f0 = k * wf, nf = win_frames(k);
         const char *o = st.dev_out[s];
         char *p = st.pin_out[s];
+        PMP_CUDA(cudaSetDevice(ln.h->device));
         for (int i = 0; i < nres; i++) {
             PMP_CUDA(cudaStreamWaitEvent(st.copy, st.computed[s][i], 0));
             if (job.values) {
@@ -434,7 +508,10 @@ int run_windows(pmp_handle *h, const WindowJob &job, pmp_report *total)
         return PMP_OK;
     };
     auto finish = [&](int k) -> int {
-        const int s = k & 1, f0 = k * wf, nf = win_frames(k);
+        Lane &ln = lanes[k % n];
+        HostStage &st = *ln.st;
+        const int s = (k / n) & 1, f0 = k * wf, nf = win_frames(k);
+        PMP_CUDA(cudaSetDevice(ln.h->device));
         PMP_CUDA(cudaEventSynchronize(st.downloaded[s]));
         const char *p = st.pin_out[s];
         pmp_window w;
@@ -463,8 +540,8 @@ int run_windows(pmp_handle *h, const WindowJob &job, pmp_report *total)
         }
         unsigned int sat;
         memcpy(&sat, p + off_sat, sizeof(sat));
-        w.report.fp16_saturation_events = (long long)(sat - sat_prev);
-        sat_prev = sat;
+        w.report.fp16_saturation_events = (long long)(sat - ln.sat_prev);
+        ln.sat_prev = sat;
         total->blocks += w.report.blocks;
         total->near_tie_blocks += w.report.near_tie_blocks;
         total->near_threshold_blocks += w.report.near_threshold_blocks;
@@ -476,20 +553,135 @@ int run_windows(pmp_handle *h, const WindowJob &job, pmp_report *total)
         return PMP_OK;
     };
 
-    rc = upload(0);
+    for (int k = 0; k < n && !rc; k++)
+        if (!(rc = upload(k))) rc = compute(k);
     for (int k = 0; k < nwin && !rc; k++) {
-        if ((rc = compute(k))) break;
-        if (k + 1 < nwin && (rc = upload(k + 1))) break;
+        if (k >= n && (rc = compute(k))) break;
+        if (k + n < nwin && (rc = upload(k + n))) break;
         if ((rc = download(k))) break;
-        if (k >= 1) rc = finish(k - 1);
+        if (k >= n) rc = finish(k - n);
     }
-    if (!rc) rc = finish(nwin - 1);
+    for (int k = std::max(0, nwin - n); k < nwin && !rc; k++) rc = finish(k);
     if (rc) {
-        cudaStreamSynchronize(st.compute);
-        cudaStreamSynchronize(st.copy);
+        for (Lane &ln : lanes) {
+            cudaSetDevice(ln.h->device);
+            cudaStreamSynchronize(ln.st->compute);
+            cudaStreamSynchronize(ln.st->copy);
+        }
         return rc;
     }
     return total->fp16_saturation_events ? saturation_error(total->fp16_saturation_events) : PMP_OK;
+}
+
+// pmp_predict_stream over `n` handles: wsets [n][n_qps][4], window k on hs[k % n].  caller >= 0 (the calling thread's
+// device): pmp_predict_stream_multi's messages, which name the handle, and its device rule, `caller` current in every
+// callback; -1: pmp_predict_stream's.
+int predict_stream(pmp_handle *const *hs, int n, int n_qps, const int *wsets, int frames, int width, int height,
+                   int sample_bytes, int window_frames, int outputs, pmp_read_cb read, pmp_write_cb write, void *user,
+                   pmp_report *report, int caller)
+{
+    const bool multi = caller >= 0;
+    if (report) memset(report, 0, sizeof(*report));
+    PMP_CHECK_ARG(n_qps >= 1 && n_qps <= 4, "n_qps must be 1 to 4");
+    PMP_CHECK_ARG(wsets != nullptr, "null wsets");
+    PMP_CHECK_ARG(read && write, "null callback");
+    PMP_CHECK_ARG(outputs != 0 && (outputs & ~(PMP_OUT_VALUES | PMP_OUT_TEXT)) == 0,
+                  "outputs must be PMP_OUT_VALUES, PMP_OUT_TEXT or both");
+    PMP_CHECK_ARG(frames >= 0 && width >= 0 && height >= 0, "negative size");
+    PMP_CHECK_ARG((width % 2) == 0 && (height % 2) == 0, "4:2:0 planes need even width and height");
+    PMP_CHECK_ARG(sample_bytes == 1 || sample_bytes == 2, "sample_bytes must be 1 or 2");
+    WindowJob job;
+    bool chroma = false;
+    for (int q = 0; q < n_qps; q++) {
+        int rc = check_wsets(hs[0], wsets + 4 * q, 4 * q, job.on[q]);
+        if (rc) {
+            if (multi) set_error("handles[0]: %s", std::string(pmp_last_error()).c_str());
+            return rc;
+        }
+        PMP_CHECK_ARG(job.on[q][0] || job.on[q][1], "both components of a QP are skipped");
+        chroma = chroma || job.on[q][1];
+    }
+    // every other handle must compute what hs[0] computes: the same skip pattern, net kinds and weights, engine and
+    // tc_dtype, and near_tol (the decode flags of the report)
+    for (int i = 1; i < n; i++) {
+        const Handle *a = hs[0], *b = hs[i];
+        const int *wa = wsets, *wb = wsets + 4 * n_qps * i;
+        auto differs = [&](const std::string &what) {
+            set_error("bad argument: handles[%d] does not compute what handles[0] computes: %s", i, what.c_str());
+            return PMP_ERR_ARG;
+        };
+        for (int q = 0; q < n_qps; q++) {
+            bool on[2];
+            int rc = check_wsets(b, wb + 4 * q, 4 * n_qps * i + 4 * q, on);
+            if (rc) {
+                set_error("handles[%d]: %s", i, std::string(pmp_last_error()).c_str());
+                return rc;
+            }
+            for (int c = 0; c < 2; c++)
+                if (on[c] != job.on[q][c])
+                    return differs(std::string(c ? "chroma" : "luma") + " of QP row " + std::to_string(q) + " is " +
+                                   (on[c] ? "run" : "skipped") + " here and " + (on[c] ? "skipped" : "run") + " there");
+            for (int k = 0; k < 4; k++) {
+                if (!on[k / 2]) continue;
+                uint64_t fa, fb;
+                if ((rc = wset_fingerprint(hs[0], wa[4 * q + k], &fa)) || (rc = wset_fingerprint(hs[i], wb[4 * q + k], &fb)))
+                    return rc;
+                if (fa != fb) {
+                    char m[160];
+                    snprintf(m, sizeof m, "the weights of wsets[%d][%d][%d] = %d (fingerprint %016llx, handles[0]'s %016llx)",
+                             i, q, k, wb[4 * q + k], (unsigned long long)fb, (unsigned long long)fa);
+                    return differs(m);
+                }
+            }
+        }
+        if (b->engine != a->engine)
+            return differs("engine " + std::to_string(b->engine) + ", handles[0]'s " + std::to_string(a->engine));
+        if (b->tc_dtype != a->tc_dtype)
+            return differs("tc_dtype " + std::to_string(b->tc_dtype) + ", handles[0]'s " + std::to_string(a->tc_dtype));
+        if (b->near_tol != a->near_tol) {
+            char m[96];
+            snprintf(m, sizeof m, "near_tol %g, handles[0]'s %g", b->near_tol, a->near_tol);
+            return differs(m);
+        }
+    }
+    const int bh = height / 64, bw = width / 64, bpf = bh * bw;
+    if (frames == 0 || bpf == 0) return PMP_OK;
+    // the default window: 4800 blocks, but small enough that every handle gets one
+    const int wf = std::min(frames, window_frames > 0 ? window_frames : std::max(1, std::min(4800 / bpf, (frames + n - 1) / n)));
+    PMP_CHECK_ARG((long long)wf * bpf < (1LL << 30) && (long long)wf * pmp_frame_values(bh, bw) <= TEXT_MAX_VALUES,
+                  "too many blocks per window");
+    job.n_qps = n_qps;
+    job.frames = frames;
+    job.width = width;
+    job.height = height;
+    job.sample_bytes = sample_bytes;
+    job.wf = wf;
+    job.values = (outputs & PMP_OUT_VALUES) != 0;
+    job.text = (outputs & PMP_OUT_TEXT) != 0;
+    job.stop_on_saturation = true;
+    job.fill = [&](int f0, int nf, char *const pin[3], const char **) -> int {
+        if (multi) PMP_CUDA(cudaSetDevice(caller));
+        const int r = read(user, f0, nf, pin[0], chroma ? pin[1] : nullptr, chroma ? pin[2] : nullptr);
+        if (r == 0) return PMP_OK;
+        set_error("the read callback returned %d for frames %d..%d", r, f0, f0 + nf - 1);
+        return PMP_ERR_ABORTED;
+    };
+    job.write = [&](const pmp_window &w) -> int {
+        if (multi) PMP_CUDA(cudaSetDevice(caller));
+        const int r = write(user, &w);
+        if (r == 0) return PMP_OK;
+        set_error("the write callback returned %d for frames %d..%d", r, w.first_frame, w.first_frame + w.frames - 1);
+        return PMP_ERR_ABORTED;
+    };
+    std::vector<Lane> lanes(n);
+    for (int i = 0; i < n; i++) {
+        lanes[i].h = hs[i];
+        lanes[i].wsets = wsets + 4 * n_qps * i;
+    }
+    pmp_report tot;
+    const int rc = run_windows(lanes, job, &tot);
+    if (report) *report = tot;
+    return rc;
 }
 
 }  // namespace
@@ -510,6 +702,7 @@ void pmp_destroy(pmp_handle *h)
 {
     if (!h) return;
     release_stage(h);
+    release_fingerprints(h);
     release_text_status(h);
     pmp_destroy_core(h);
 }
@@ -547,7 +740,6 @@ int pmp_predict_host(pmp_handle *h, const int wsets[4], const void *y, const voi
     PMP_CHECK_ARG(pitch_y >= row_y && pitch_c >= row_c, "pitch smaller than a row");
     if (chunk <= 0) chunk = 4800;
     job.n_qps = 1;
-    memcpy(job.wsets[0], wsets, sizeof(job.wsets[0]));
     job.frames = frames;
     job.width = width;
     job.height = height;
@@ -584,8 +776,11 @@ int pmp_predict_host(pmp_handle *h, const int wsets[4], const void *y, const voi
             if (on[c] && !direct_out[c]) memcpy(outs[c] + (size_t)w.first_frame * per, w.values[0][c], (size_t)w.n_values[0][c]);
         return PMP_OK;
     };
+    std::vector<Lane> lanes(1);
+    lanes[0].h = h;
+    lanes[0].wsets = wsets;
     pmp_report tot;
-    rc = run_windows(h, job, &tot);
+    rc = run_windows(lanes, job, &tot);
     if (report && (rc == PMP_OK || rc == PMP_ERR_STATE)) *report = tot;
     return rc;
 }
@@ -608,53 +803,30 @@ int pmp_predict_stream(pmp_handle *h, int n_qps, const int *wsets, int frames, i
                        pmp_report *report)
 {
     H_CHECK(h);
+    return predict_stream(&h, 1, n_qps, wsets, frames, width, height, sample_bytes, window_frames, outputs, read, write,
+                          user, report, -1);
+}
+
+int pmp_predict_stream_multi(pmp_handle *const *handles, int n_handles, int n_qps, const int *wsets, int frames,
+                             int width, int height, int sample_bytes, int window_frames, int outputs, pmp_read_cb read,
+                             pmp_write_cb write, void *user, pmp_report *report)
+{
     if (report) memset(report, 0, sizeof(*report));
-    PMP_CHECK_ARG(n_qps >= 1 && n_qps <= 4, "n_qps must be 1 to 4");
-    PMP_CHECK_ARG(wsets != nullptr, "null wsets");
-    PMP_CHECK_ARG(read && write, "null callback");
-    PMP_CHECK_ARG(outputs != 0 && (outputs & ~(PMP_OUT_VALUES | PMP_OUT_TEXT)) == 0,
-                  "outputs must be PMP_OUT_VALUES, PMP_OUT_TEXT or both");
-    PMP_CHECK_ARG(frames >= 0 && width >= 0 && height >= 0, "negative size");
-    PMP_CHECK_ARG((width % 2) == 0 && (height % 2) == 0, "4:2:0 planes need even width and height");
-    PMP_CHECK_ARG(sample_bytes == 1 || sample_bytes == 2, "sample_bytes must be 1 or 2");
-    WindowJob job;
-    bool chroma = false;
-    for (int q = 0; q < n_qps; q++) {
-        int rc = check_wsets(h, wsets + 4 * q, 4 * q, job.on[q]);
-        if (rc) return rc;
-        PMP_CHECK_ARG(job.on[q][0] || job.on[q][1], "both components of a QP are skipped");
-        memcpy(job.wsets[q], wsets + 4 * q, sizeof(job.wsets[q]));
-        chroma = chroma || job.on[q][1];
+    PMP_CHECK_ARG(n_handles >= 1 && n_handles <= STREAM_HANDLES_MAX, "n_handles must be 1 to 16");
+    PMP_CHECK_ARG(handles != nullptr, "null handles");
+    for (int i = 0; i < n_handles; i++) {
+        if (!handles[i]) { set_error("bad argument: handles[%d] is null", i); return PMP_ERR_ARG; }
+        for (int j = 0; j < i; j++)
+            if (handles[j] == handles[i]) {
+                set_error("bad argument: handles[%d] is handles[%d]: every handle must be distinct", i, j);
+                return PMP_ERR_ARG;
+            }
     }
-    const int bh = height / 64, bw = width / 64, bpf = bh * bw;
-    if (frames == 0 || bpf == 0) return PMP_OK;
-    const int wf = std::min(frames, window_frames > 0 ? window_frames : std::max(1, 4800 / bpf));
-    PMP_CHECK_ARG((long long)wf * bpf < (1LL << 30) && (long long)wf * pmp_frame_values(bh, bw) <= TEXT_MAX_VALUES,
-                  "too many blocks per window");
-    job.n_qps = n_qps;
-    job.frames = frames;
-    job.width = width;
-    job.height = height;
-    job.sample_bytes = sample_bytes;
-    job.wf = wf;
-    job.values = (outputs & PMP_OUT_VALUES) != 0;
-    job.text = (outputs & PMP_OUT_TEXT) != 0;
-    job.stop_on_saturation = true;
-    job.fill = [&](int f0, int nf, char *const pin[3], const char **) -> int {
-        const int r = read(user, f0, nf, pin[0], chroma ? pin[1] : nullptr, chroma ? pin[2] : nullptr);
-        if (r == 0) return PMP_OK;
-        set_error("the read callback returned %d for frames %d..%d", r, f0, f0 + nf - 1);
-        return PMP_ERR_ABORTED;
-    };
-    job.write = [&](const pmp_window &w) -> int {
-        const int r = write(user, &w);
-        if (r == 0) return PMP_OK;
-        set_error("the write callback returned %d for frames %d..%d", r, w.first_frame, w.first_frame + w.frames - 1);
-        return PMP_ERR_ABORTED;
-    };
-    pmp_report tot;
-    const int rc = run_windows(h, job, &tot);
-    if (report) *report = tot;
+    int caller = 0;
+    PMP_CUDA(cudaGetDevice(&caller));
+    const int rc = predict_stream(handles, n_handles, n_qps, wsets, frames, width, height, sample_bytes, window_frames,
+                                  outputs, read, write, user, report, caller);
+    cudaSetDevice(caller);
     return rc;
 }
 

@@ -1,8 +1,8 @@
 // pmp_predict: PartitionMat files from a YUV sequence without Python (C++11; include/pmp_b200.h + libpmp_b200.so only).
 //
 //   pmp_predict --input SEQ.yuv --width W --height H --frames N [--bitDepth 8|10] [--ssRatio S] [--qps 22,27,32,37]
-//               --modelDir DIR --outDir DIR [--binaryOut] [--device D] [--tcDtype fp16|bf16] [--chunk C] [--timing]
-//               [--stream]
+//               --modelDir DIR --outDir DIR [--binaryOut] [--device D | --devices D,D,...] [--tcDtype fp16|bf16]
+//               [--chunk C] [--timing] [--stream]
 //
 // The weights are the exported .pmpw files (python -m pmp_vvc_tip2023_b200.export_weights): <comp>_Q_<qp>.pmpw and
 // <comp>_BD_<qp>.pmpw in --modelDir.  Frames are read as Inference_QBD.import_yuv420 reads them (every S-th frame, by
@@ -18,6 +18,10 @@
 // <stem>.txt.part (.bin.part) while the next window computes; the .part files are renamed once the call succeeds and
 // deleted otherwise, so existing files are left as they were.  Host memory is bounded by the window (--chunk blocks,
 // default 4800), not by the sequence.  The files are the same as without --stream.
+//
+// --devices D,D,... (with --stream) creates one handle per entry, each loading the same weight files, and makes one
+// pmp_predict_stream_multi call: window k runs on the (k mod n)-th handle while the files are written in frame order.
+// Entries may repeat (--devices 0,0: two handles on GPU 0).  A single entry without --stream is --device.
 #include "pmp_b200.h"
 
 #include <chrono>
@@ -34,14 +38,15 @@ struct Args {
     std::string input, model_dir, out_dir;
     int width = 0, height = 0, frames = 0, bit_depth = 8, ss_ratio = 1, device = 0, chunk = 0;
     std::vector<int> qps{22, 27, 32, 37};
-    bool binary_out = false, bf16 = false, timing = false, stream = false;
+    std::vector<int> devices;       // --devices; empty: the one handle on --device
+    bool binary_out = false, bf16 = false, timing = false, stream = false, device_given = false;
 };
 
 int usage(const char *msg)
 {
     std::fprintf(stderr,
                  "pmp_predict: %s\nusage: pmp_predict --input SEQ.yuv --width W --height H --frames N [--bitDepth 8|10] "
-                 "[--ssRatio S] [--qps 22,27,32,37] --modelDir DIR --outDir DIR [--binaryOut] [--device D] "
+                 "[--ssRatio S] [--qps 22,27,32,37] --modelDir DIR --outDir DIR [--binaryOut] [--device D | --devices D,D,...] "
                  "[--tcDtype fp16|bf16] [--chunk C] [--timing] [--stream]\n",
                  msg);
     return 2;
@@ -64,7 +69,21 @@ bool parse(int argc, char **argv, Args &a, std::string &err)
         else if (k == "--frames") a.frames = std::atoi(v.c_str());
         else if (k == "--bitDepth") a.bit_depth = std::atoi(v.c_str());
         else if (k == "--ssRatio") a.ss_ratio = std::atoi(v.c_str());
-        else if (k == "--device") a.device = std::atoi(v.c_str());
+        else if (k == "--device") { a.device = std::atoi(v.c_str()); a.device_given = true; }
+        else if (k == "--devices") {
+            a.devices.clear();
+            for (size_t p = 0; p <= v.size();) {
+                size_t q = v.find(',', p);
+                if (q == std::string::npos) q = v.size();
+                const std::string d = v.substr(p, q - p);
+                if (d.empty() || d.size() > 4 || d.find_first_not_of("0123456789") != std::string::npos) {
+                    err = "--devices takes comma-separated device numbers, got '" + v + "'";
+                    return false;
+                }
+                a.devices.push_back(std::atoi(d.c_str()));
+                p = q + 1;
+            }
+        }
         else if (k == "--chunk") a.chunk = std::atoi(v.c_str());
         else if (k == "--tcDtype") {
             if (v != "fp16" && v != "bf16") { err = "--tcDtype must be fp16 or bf16"; return false; }
@@ -88,6 +107,9 @@ bool parse(int argc, char **argv, Args &a, std::string &err)
     if (a.width <= 0 || a.height <= 0 || a.frames <= 0 || a.width % 2 || a.height % 2) { err = "bad --width/--height/--frames"; return false; }
     if (a.bit_depth != 8 && a.bit_depth != 10) { err = "--bitDepth must be 8 or 10"; return false; }
     if (a.ss_ratio < 1) { err = "--ssRatio must be at least 1"; return false; }
+    if (a.device_given && !a.devices.empty()) { err = "--device and --devices exclude each other"; return false; }
+    if (a.devices.size() > 1 && !a.stream) { err = "--devices with more than one device needs --stream"; return false; }
+    if (a.devices.size() > 16) { err = "--devices takes at most 16 entries"; return false; }
     return true;
 }
 
@@ -206,7 +228,8 @@ int stream_write(void *user, const pmp_window *w)
     return 0;
 }
 
-int run_stream(const Args &a, pmp_handle *h, const std::vector<int> &wsets, const std::string &base)
+// hs: the one handle of pmp_predict_stream, or with --devices the handles of pmp_predict_stream_multi; wsets: [handle][qp][4]
+int run_stream(const Args &a, const std::vector<pmp_handle *> &hs, const std::vector<int> &wsets, const std::string &base)
 {
     Stream st;
     st.a = &a;
@@ -242,11 +265,20 @@ int run_stream(const Args &a, pmp_handle *h, const std::vector<int> &wsets, cons
     if (ok) {
         const auto t0 = std::chrono::steady_clock::now();
         const int window = a.chunk > 0 && bpf > 0 ? std::max(1, a.chunk / bpf) : 0;
-        rc = pmp_predict_stream(h, (int)a.qps.size(), wsets.data(), nf, a.width, a.height, st.sb, window,
-                                PMP_OUT_TEXT | (a.binary_out ? PMP_OUT_VALUES : 0), stream_read, stream_write, &st, &tot);
+        const int outputs = PMP_OUT_TEXT | (a.binary_out ? PMP_OUT_VALUES : 0), n = (int)hs.size();
+        if (a.devices.empty())
+            rc = pmp_predict_stream(hs[0], (int)a.qps.size(), wsets.data(), nf, a.width, a.height, st.sb, window, outputs,
+                                    stream_read, stream_write, &st, &tot);
+        else
+            rc = pmp_predict_stream_multi(hs.data(), n, (int)a.qps.size(), wsets.data(), nf, a.width, a.height, st.sb,
+                                          window, outputs, stream_read, stream_write, &st, &tot);
         const double ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-        const int wf = window > 0 ? window : std::max(1, bpf > 0 ? 4800 / bpf : 1);
-        if (a.timing) std::printf("pmp_predict_stream %.3f ms (%d frames, %d windows)\n", ms, nf, bpf > 0 ? (nf + wf - 1) / wf : 0);
+        const int wf = window > 0 ? window : std::max(1, bpf > 0 ? std::min(4800 / bpf, (nf + n - 1) / n) : 1);
+        if (a.timing && a.devices.empty())
+            std::printf("pmp_predict_stream %.3f ms (%d frames, %d windows)\n", ms, nf, bpf > 0 ? (nf + wf - 1) / wf : 0);
+        else if (a.timing)
+            std::printf("pmp_predict_stream_multi %.3f ms (%d frames, %d windows, %d handles)\n", ms, nf,
+                        bpf > 0 ? (nf + wf - 1) / wf : 0, n);
     }
     std::fclose(st.in);
     for (size_t i = 0; i < st.txt.size(); i++) {
@@ -276,6 +308,28 @@ int run_stream(const Args &a, pmp_handle *h, const std::vector<int> &wsets, cons
     return 1;
 }
 
+// A handle on `device` with every QP's weight sets from --modelDir appended to wsets ([qp][4]); nullptr after a message.
+pmp_handle *open_handle(const Args &a, int device, std::vector<int> &wsets)
+{
+    static const char *const comps[2] = {"Luma", "Chroma"};
+    pmp_handle *h = nullptr;
+    if (pmp_create(device, &h) != PMP_OK) { fail("pmp_create"); return nullptr; }
+    if (pmp_set_engine(h, PMP_ENGINE_TC, a.bf16 ? PMP_TC_BF16 : PMP_TC_FP16) != PMP_OK) { fail("pmp_set_engine"); return nullptr; }
+    for (size_t q = 0; q < a.qps.size(); q++)
+        for (int c = 0; c < 2; c++)
+            for (int k = 0; k < 2; k++) {
+                const std::string path = a.model_dir + "/" + comps[c] + (k ? "_BD_" : "_Q_") + std::to_string(a.qps[q]) + ".pmpw";
+                int net = -1, ws = -1;
+                if (pmp_weights_load(h, path.c_str(), &net, &ws) != PMP_OK) { fail("pmp_weights_load"); return nullptr; }
+                if (net != 2 * c + k) {
+                    std::fprintf(stderr, "pmp_predict: %s holds net kind %d, expected %d\n", path.c_str(), net, 2 * c + k);
+                    return nullptr;
+                }
+                wsets.push_back(ws);
+            }
+    return h;
+}
+
 }  // namespace
 
 int main(int argc, char **argv)
@@ -283,30 +337,21 @@ int main(int argc, char **argv)
     Args a;
     std::string err;
     if (!parse(argc, argv, a, err)) return usage(err.c_str());
-    pmp_handle *h = nullptr;
-    if (pmp_create(a.device, &h) != PMP_OK) return fail("pmp_create");
-    int rc = pmp_set_engine(h, PMP_ENGINE_TC, a.bf16 ? PMP_TC_BF16 : PMP_TC_FP16);
-    if (rc) return fail("pmp_set_engine");
-
-    const char *const comps[2] = {"Luma", "Chroma"};
-    std::vector<int> wsets(4 * a.qps.size());
-    for (size_t q = 0; q < a.qps.size(); q++)
-        for (int c = 0; c < 2; c++)
-            for (int k = 0; k < 2; k++) {
-                const std::string path = a.model_dir + "/" + comps[c] + (k ? "_BD_" : "_Q_") + std::to_string(a.qps[q]) + ".pmpw";
-                int net = -1;
-                if (pmp_weights_load(h, path.c_str(), &net, &wsets[4 * q + 2 * c + k]) != PMP_OK) return fail("pmp_weights_load");
-                if (net != 2 * c + k) {
-                    std::fprintf(stderr, "pmp_predict: %s holds net kind %d, expected %d\n", path.c_str(), net, 2 * c + k);
-                    return 1;
-                }
-            }
+    if (a.devices.size() == 1 && !a.stream) a.device = a.devices[0];
+    std::vector<pmp_handle *> hs;
+    std::vector<int> wsets;         // [handle][qp][4]
+    for (int d : (a.stream && !a.devices.empty()) ? a.devices : std::vector<int>{a.device}) {
+        hs.push_back(open_handle(a, d, wsets));
+        if (!hs.back()) return 1;
+    }
+    pmp_handle *h = hs[0];
+    int rc;
 
     std::string base = a.input.substr(a.input.find_last_of('/') + 1);
     if (base.size() > 4 && base.compare(base.size() - 4, 4, ".yuv") == 0) base.resize(base.size() - 4);
     if (a.stream) {
-        rc = run_stream(a, h, wsets, base);
-        pmp_destroy(h);
+        rc = run_stream(a, hs, wsets, base);
+        for (pmp_handle *x : hs) pmp_destroy(x);
         return rc;
     }
 
