@@ -240,6 +240,25 @@ int pmp_predict_stream_multi(pmp_handle *const *handles, int n_handles, int n_qp
                              int width, int height, int sample_bytes, int window_frames, int outputs, pmp_read_cb read,
                              pmp_write_cb write, void *user, pmp_report *report);
 
+/* pmp_predict_stream_ex: pmp_predict_stream_multi where a row is a pair (weight sets, decode thresholds) instead of a QP,
+ * so that one call writes PartitionMat data under several threshold settings of Map_to_Partition (Map2Partition.py:100),
+ * or several QPs under several settings.
+ * n_rows: 1..4; wsets: [n_handles][n_rows][4] as pmp_predict_stream_multi's; lamb: [n_rows][5] doubles, row r's lamb1..lamb5
+ * (NULL: the reference defaults 0.7, 0.7, 1.5, 0.3, 0.7 for every row).  A threshold that is not finite returns
+ * PMP_ERR_ARG before any callback; the message names the row and the index.  w->values/text[r][c] and w->n_qps (= n_rows)
+ * of pmp_window refer to rows; w->report counts each row's blocks, and its near-tie count (flags bit 0) depends on the
+ * row's thresholds.
+ * Rows of a handle whose (Q, MSBD) weight-set ids for a component are equal share that component's net pass: per window
+ * and chunk, pmp_predict_maps and pmp_qt_postprocess run once, then pmp_map2partition_ex and pmp_assemble_frames run once
+ * per row.  Four settings of one QP cost one net pass per window plus four decodes, assemblies and texts.
+ * Everything else (callbacks, consistency check across handles, errors, saturation stop, report, bounded staging, every
+ * return leaving no work queued) is pmp_predict_stream_multi's.  With lamb NULL, or rows equal to the defaults, the output
+ * is byte-identical to pmp_predict_stream_multi on the same arguments; pmp_predict_stream_multi is this call with
+ * lamb NULL. */
+int pmp_predict_stream_ex(pmp_handle *const *handles, int n_handles, int n_rows, const int *wsets, const double *lamb,
+                          int frames, int width, int height, int sample_bytes, int window_frames, int outputs,
+                          pmp_read_cb read, pmp_write_cb write, void *user, pmp_report *report);
+
 /* Self-test of the TC conv engine against the SIMT engine on random data (GPU).  Returns 0 and the
  * max-abs error in *max_err, or an error.  flags: bit0 ReLU, bit1 identity residual, bit2 attention product,
  * bit3 bf16 operands; kernel variants: bits 8..9 accumulator scheme of the single-CTA kernel (1 unstacked, 2 stacked),

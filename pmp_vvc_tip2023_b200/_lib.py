@@ -75,6 +75,8 @@ SIGNATURES = {
                                    c_void_p, _P(Report)]),
     "pmp_predict_stream_multi": (c_int, [_P(c_void_p), c_int, c_int, _P(c_int), c_int, c_int, c_int, c_int, c_int, c_int,
                                          READ_CB, WRITE_CB, c_void_p, _P(Report)]),
+    "pmp_predict_stream_ex": (c_int, [_P(c_void_p), c_int, c_int, _P(c_int), _P(ctypes.c_double), c_int, c_int, c_int, c_int,
+                                      c_int, c_int, READ_CB, WRITE_CB, c_void_p, _P(Report)]),
     "pmp_cut_blocks": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p,
                                c_void_p]),
     "pmp_run_component": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int, c_int, c_int, c_void_p,
@@ -238,13 +240,18 @@ class Handle:
         return res
 
     def predict_stream(self, wsets_by_qp, frames, width, height, sample_bytes, read, write, window_frames=0,
-                       outputs=OUT_VALUES | OUT_TEXT, report=None):
+                       outputs=OUT_VALUES | OUT_TEXT, report=None, lamb=None):
         """pmp_predict_stream.  wsets_by_qp: one (luma Q, luma MSBD, chroma Q, chroma MSBD) row per QP (1 to 4 rows).
         read(first_frame, frames, y, u, v) fills numpy views of the library's page-locked planes: y [frames, H, W],
         u/v [frames, H/2, W/2] (None when no QP runs chroma), uint8 or uint16 after sample_bytes.
         write(w) receives a StreamWindow per window, in frame order; its arrays are views valid only during the call.
         A non-zero return of a callback aborts the call (PmpError, error -6); an exception raised in a callback aborts
-        it too and is re-raised here, chained to that error.  Returns the Report summed over the windows written."""
+        it too and is re-raised here, chained to that error.  Returns the Report summed over the windows written.
+        lamb: None, or one (lamb1..lamb5) decode-threshold tuple per row (pmp_predict_stream_ex on this handle); rows with
+        equal weight sets share their net pass."""
+        if lamb is not None:
+            return predict_stream_multi([self], [wsets_by_qp], frames, width, height, sample_bytes, read, write,
+                                        window_frames, outputs, report, lamb)
         rows = [list(r) for r in wsets_by_qp]
         flat = (c_int * (4 * max(len(rows), 1)))(*[w for r in rows for w in r])
         return _stream_call(lambda rd, wr, rep: lib().pmp_predict_stream(
@@ -253,11 +260,13 @@ class Handle:
 
 
 def predict_stream_multi(handles, wsets_by_handle, frames, width, height, sample_bytes, read, write, window_frames=0,
-                         outputs=OUT_VALUES | OUT_TEXT, report=None):
+                         outputs=OUT_VALUES | OUT_TEXT, report=None, lamb=None):
     """pmp_predict_stream_multi: Handle.predict_stream over several handles (1 to 16, on one or several devices), window
     k on handles[k % len(handles)].  wsets_by_handle[i]: handles[i]'s rows, one (luma Q, luma MSBD, chroma Q,
     chroma MSBD) per QP, the same QPs and weights on every handle.  The callbacks, errors and result are those of
-    Handle.predict_stream; the calling thread's current device is current inside the callbacks and after the call."""
+    Handle.predict_stream; the calling thread's current device is current inside the callbacks and after the call.
+    lamb: None, or one (lamb1..lamb5) decode-threshold tuple per row (pmp_predict_stream_ex): row r's results are
+    decoded with lamb[r]; a wrong length raises ValueError before the library is called."""
     nh = len(handles)
     rows = [[list(r) for r in by_qp] for by_qp in wsets_by_handle]
     nq = len(rows[0]) if rows else 0
@@ -265,9 +274,17 @@ def predict_stream_multi(handles, wsets_by_handle, frames, width, height, sample
         raise ValueError("wsets_by_handle needs one list of %d QP rows per handle" % nq)
     flat = (c_int * (4 * max(nh * nq, 1)))(*[w for by_qp in rows for r in by_qp for w in r])
     hs = (c_void_p * max(nh, 1))(*[h.ptr if isinstance(h, Handle) else h for h in handles])
-    return _stream_call(lambda rd, wr, rep: lib().pmp_predict_stream_multi(
-        hs, nh, nq, flat, int(frames), int(width), int(height), int(sample_bytes), int(window_frames), int(outputs), rd,
-        wr, None, rep), width, height, sample_bytes, read, write, report)
+    if lamb is None:
+        return _stream_call(lambda rd, wr, rep: lib().pmp_predict_stream_multi(
+            hs, nh, nq, flat, int(frames), int(width), int(height), int(sample_bytes), int(window_frames), int(outputs),
+            rd, wr, None, rep), width, height, sample_bytes, read, write, report)
+    lamb = [tuple(t) for t in lamb]
+    if len(lamb) != nq or any(len(t) != 5 for t in lamb):
+        raise ValueError("lamb needs one (lamb1, lamb2, lamb3, lamb4, lamb5) tuple per row: %d rows" % nq)
+    lam = (ctypes.c_double * (5 * max(nq, 1)))(*[float(x) for t in lamb for x in t])
+    return _stream_call(lambda rd, wr, rep: lib().pmp_predict_stream_ex(
+        hs, nh, nq, flat, lam, int(frames), int(width), int(height), int(sample_bytes), int(window_frames),
+        int(outputs), rd, wr, None, rep), width, height, sample_bytes, read, write, report)
 
 
 def _stream_call(call, width, height, sample_bytes, read, write, report):

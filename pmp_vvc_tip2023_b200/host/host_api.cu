@@ -1,8 +1,9 @@
 // Host-level entry points of libpmp_b200 for callers without Python or CUDA of their own (include/pmp_b200.h):
 // pmp_weights_load (exported .pmpw weight files), pmp_predict_host (host planes in, host PartitionMat vectors out),
 // pmp_predict_stream (frames in through a callback, every QP's vectors and text out window by window),
-// pmp_predict_stream_multi (the same over several handles, windows in rotation) and pmp_format_texts (text_batch.cu), plus pmp_destroy, which releases this layer's staging before the core handle
-// teardown in csrc/api.cu.
+// pmp_predict_stream_multi (the same over several handles, windows in rotation), pmp_predict_stream_ex (the same with
+// decode thresholds per row) and pmp_format_texts (text_batch.cu), plus pmp_destroy, which releases this layer's staging
+// before the core handle teardown in csrc/api.cu.
 //
 // This layer only calls the core's entry points and internal functions; it lives outside csrc/ because bench.py ties
 // the committed ncu traffic summary (profiles/r*_traffic.json) to a hash of the csrc/ sources, and none of those kernels
@@ -12,6 +13,7 @@
 
 #include <algorithm>
 #include <climits>
+#include <cmath>
 #include <cstdio>
 #include <cstring>
 #include <functional>
@@ -159,12 +161,13 @@ int weights_load(Handle *h, const char *path, int *net_out, int *wset)
     return rc;
 }
 
-// ---- the window pipeline of pmp_predict_host, pmp_predict_stream and pmp_predict_stream_multi ---------------------
-// Per handle: a compute and a copy stream, their events, and per window slot (double-buffered) pinned + device buffers
-// for the input planes and for the results (values, decode flags and, when asked for, text of every (QP, component)
-// pair, the text byte counts and a snapshot of the saturation counter).  Created on first use, grown to the largest
-// window, released by pmp_destroy.
-constexpr int RESULTS_MAX = 8;      // 4 QPs x 2 components
+// ---- the window pipeline of pmp_predict_host, pmp_predict_stream, pmp_predict_stream_multi and _ex ----------------
+// Per handle: a compute and a copy stream, their events, per window slot (double-buffered) pinned + device buffers for
+// the input planes and for the results (values, decode flags and, when asked for, text of every (row, component) pair,
+// the text byte counts and a snapshot of the saturation counter), and, used by the compute stream only, the cut blocks
+// and the work area of the per-window schedule (one chunk's float maps, the post-processed qt map and each row's decoded
+// integer maps).  Created on first use, grown to the largest window, released by pmp_destroy.
+constexpr int RESULTS_MAX = 8;      // 4 rows x 2 components
 constexpr int STREAM_HANDLES_MAX = 16;     // handles of one pmp_predict_stream_multi call
 
 struct HostStage {
@@ -172,7 +175,8 @@ struct HostStage {
     cudaEvent_t uploaded[2] = {}, cut[2] = {}, finished[2] = {}, downloaded[2] = {}, computed[2][RESULTS_MAX] = {};
     char *pin_in[2] = {}, *pin_out[2] = {}, *dev_in[2] = {}, *dev_out[2] = {};
     uint8_t *dev_blocks = nullptr;
-    size_t in_bytes = 0, out_bytes = 0, blocks_bytes = 0;     // per slot
+    char *dev_work = nullptr;
+    size_t in_bytes = 0, out_bytes = 0, blocks_bytes = 0, work_bytes = 0;     // in, out: per slot
 };
 
 std::mutex g_stage_mu;
@@ -204,21 +208,26 @@ void free_buffers(HostStage &st)
         st.pin_in[s] = st.pin_out[s] = st.dev_in[s] = st.dev_out[s] = nullptr;
     }
     if (st.dev_blocks) cudaFree(st.dev_blocks);
+    if (st.dev_work) cudaFree(st.dev_work);
     st.dev_blocks = nullptr;
-    st.in_bytes = st.out_bytes = st.blocks_bytes = 0;
+    st.dev_work = nullptr;
+    st.in_bytes = st.out_bytes = st.blocks_bytes = st.work_bytes = 0;
 }
 
-int ensure_stage(HostStage &st, size_t in_bytes, size_t out_bytes, size_t blocks_bytes)
+int ensure_stage(HostStage &st, size_t in_bytes, size_t out_bytes, size_t blocks_bytes, size_t work_bytes)
 {
     if (!st.compute) {
         PMP_CUDA(cudaStreamCreateWithFlags(&st.compute, cudaStreamNonBlocking));
         PMP_CUDA(cudaStreamCreateWithFlags(&st.copy, cudaStreamNonBlocking));
         for (cudaEvent_t *e : events_of(st)) PMP_CUDA(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
     }
-    if (in_bytes <= st.in_bytes && out_bytes <= st.out_bytes && blocks_bytes <= st.blocks_bytes) return PMP_OK;
+    if (in_bytes <= st.in_bytes && out_bytes <= st.out_bytes && blocks_bytes <= st.blocks_bytes &&
+        work_bytes <= st.work_bytes)
+        return PMP_OK;
     in_bytes = std::max(in_bytes, st.in_bytes);
     out_bytes = std::max(out_bytes, st.out_bytes);
     blocks_bytes = std::max(blocks_bytes, st.blocks_bytes);
+    work_bytes = std::max(work_bytes, st.work_bytes);
     free_buffers(st);       // the previous call ended synchronised: nothing in flight uses them
     for (int s = 0; s < 2; s++) {
         PMP_CUDA(cudaHostAlloc((void **)&st.pin_in[s], in_bytes, cudaHostAllocDefault));
@@ -227,9 +236,11 @@ int ensure_stage(HostStage &st, size_t in_bytes, size_t out_bytes, size_t blocks
         PMP_CUDA(cudaMalloc((void **)&st.dev_out[s], out_bytes));
     }
     PMP_CUDA(cudaMalloc((void **)&st.dev_blocks, blocks_bytes));
+    PMP_CUDA(cudaMalloc((void **)&st.dev_work, work_bytes));
     st.in_bytes = in_bytes;
     st.out_bytes = out_bytes;
     st.blocks_bytes = blocks_bytes;
+    st.work_bytes = work_bytes;
     return PMP_OK;
 }
 
@@ -330,11 +341,13 @@ void release_fingerprints(const Handle *h)
     g_fingerprint.erase(g_fingerprint.lower_bound({h, INT_MIN}), g_fingerprint.upper_bound({h, INT_MAX}));
 }
 
-// One call's work: the (QP, component) results over `frames` frames, in windows of `wf` whole frames.  The entry point
-// supplies the host ends of a window: fill() provides its input planes, write() takes its results.
+// One call's work: the (row, component) results over `frames` frames, in windows of `wf` whole frames.  A row is a QP's
+// weight sets and a set of decode thresholds.  The entry point supplies the host ends of a window: fill() provides its
+// input planes, write() takes its results.
 struct WindowJob {
-    int n_qps = 0, frames = 0, width = 0, height = 0, sample_bytes = 1, wf = 1, chunk = 4800;
+    int n_qps = 0, frames = 0, width = 0, height = 0, sample_bytes = 1, wf = 1, chunk = 4800;     // n_qps: the rows
     bool on[4][2] = {};
+    const double *lamb = nullptr;           // [n_qps][5] lamb1..lamb5 per row; nullptr: the reference defaults
     bool values = true, text = false;       // download the values; format and download the text
     bool stop_on_saturation = false;        // stop after the first window with saturation events, or finish them all
     bool direct_in = false;                 // fill() points src at the caller's page-locked planes and leaves pin alone
@@ -349,7 +362,7 @@ struct WindowJob {
 // One handle's part of a call: windows k with k % lanes == its index, on its own streams and staging.
 struct Lane {
     pmp_handle *h = nullptr;
-    const int *wsets = nullptr;     // [n_qps][4]: this handle's weight-set ids
+    const int *wsets = nullptr;     // [rows][4]: this handle's weight-set ids
     HostStage *st = nullptr;        // set by run_windows
     unsigned int sat_prev = 0;      // the handle's saturation counter after its previous window
 };
@@ -358,7 +371,10 @@ struct Lane {
 // uploads window k + n, downloads window k and writes window k - n, so each lane keeps both its window slots busy while
 // the host reads and writes in frame order; with one lane, window k+1 is filled and uploaded and window k-1 written
 // while window k computes.  Each lane's first window is computed as soon as it is uploaded, so that no device waits for
-// the other lanes' first reads.  Each window is cut into blocks once for all its results.  The host waits only on
+// the other lanes' first reads.  Each window is cut into blocks once for all its results.  Per component, rows whose
+// (Q, MSBD) weight-set ids are equal share one net pass: per chunk of job.chunk blocks, pmp_predict_maps and
+// pmp_qt_postprocess run once and pmp_map2partition_ex once per row with the row's thresholds; then pmp_assemble_frames
+// runs once per row.  With one row per pass this is exactly the sequence of pmp_run_component.  The host waits only on
 // events of finished windows.  The device of a lane is made current before each of its CUDA calls; fill() and write()
 // may switch devices.  *total receives the sum of the reports of the windows written.  Every return leaves no work
 // queued on any lane.
@@ -398,6 +414,11 @@ int run_windows(std::vector<Lane> &lanes, const WindowJob &job, pmp_report *tota
     }
     const size_t off_nbytes = off, off_sat = off + 8 * RESULTS_MAX;
     const size_t blk_bytes[2] = {(size_t)68 * 68, (size_t)3 * 34 * 34};
+    // the work area: one chunk's float maps (qt [64] | bt [768] | dire [768] f32 per block), the window's
+    // post-processed qt map [64] u8 per block, and per row of a shared net pass hor [256] | ver [256] | dire [768]
+    const int chunk = (int)std::min<long long>(job.chunk, nmax);
+    const size_t maps_bytes = r256((size_t)chunk * (64 + 768 + 768) * sizeof(float)), qt8_bytes = r256((size_t)nmax * 64),
+                 row_bytes = r256((size_t)nmax * (256 + 256 + 768));
     const int nwin = (frames + wf - 1) / wf;
     if ((int)lanes.size() > nwin) lanes.resize(nwin);       // lanes without a window stay untouched
     const int n = (int)lanes.size();
@@ -407,10 +428,11 @@ int run_windows(std::vector<Lane> &lanes, const WindowJob &job, pmp_report *tota
         PMP_CUDA(cudaSetDevice(h->device));
         ln.st = &stage_of(h);
         rc = ensure_stage(*ln.st, (size_t)wf * in_frame, off_sat + 256,
-                          (size_t)nmax * ((comp_on[0] ? blk_bytes[0] : 0) + (comp_on[1] ? blk_bytes[1] : 0)));
+                          (size_t)nmax * ((comp_on[0] ? blk_bytes[0] : 0) + (comp_on[1] ? blk_bytes[1] : 0)),
+                          maps_bytes + qt8_bytes + (size_t)job.n_qps * row_bytes);
         if (rc) return rc;
         // The status word and the text status words exist before the loop (allocating them synchronises the device).
-        // The arena and scratch grow inside the first window's pmp_run_component when a handle first sees this window
+        // The activation arena grows inside the first window's pmp_predict_maps when a handle first sees this chunk
         // size; that synchronises the device once and leaves everything queued intact.
         if ((rc = ensure_status(h))) return rc;
         if (job.text && (rc = reserve_text_status(h, nres, (long long)wf * per))) return rc;
@@ -458,13 +480,47 @@ int run_windows(std::vector<Lane> &lanes, const WindowJob &job, pmp_report *tota
                            job.sample_bytes, nf, job.width, job.height, blk[0], blk[1], st.compute);
         if (r) return r;
         PMP_CUDA(cudaEventRecord(st.cut[s], st.compute));
+        const long long N = (long long)nf * bpf;
+        float *cqt = (float *)st.dev_work, *cbt = cqt + (size_t)chunk * 64, *cdi = cbt + (size_t)chunk * 768;
+        uint8_t *qt8 = (uint8_t *)st.dev_work + maps_bytes;
+        bool done[RESULTS_MAX] = {};
         for (int i = 0; i < nres; i++) {
-            const int *ws = ln.wsets + 4 * res_q[i], c = res_c[i];
-            r = pmp_run_component(h, ws[2 * c], ws[2 * c + 1], c == 0, blk[c], nf, bh, bw, job.chunk,
-                                  (int8_t *)(o + off_vals[i]), nullptr, nullptr, nullptr, (uint32_t *)(o + off_flags[i]),
-                                  st.compute);
-            if (r) return r;
-            PMP_CUDA(cudaEventRecord(st.computed[s][i], st.compute));
+            if (done[i]) continue;
+            // the results that share result i's net pass: the same component and the same (Q, MSBD) weight sets
+            const int c = res_c[i], wq = ln.wsets[4 * res_q[i] + 2 * c], wb = ln.wsets[4 * res_q[i] + 2 * c + 1];
+            int grp[RESULTS_MAX], ng = 0;
+            for (int j = i; j < nres; j++) {
+                const int *wj = ln.wsets + 4 * res_q[j];
+                if (!done[j] && res_c[j] == c && wj[2 * c] == wq && wj[2 * c + 1] == wb) {
+                    grp[ng++] = j;
+                    done[j] = true;
+                }
+            }
+            auto dec = [&](int g) { return (uint8_t *)st.dev_work + maps_bytes + qt8_bytes + (size_t)g * row_bytes; };
+            for (long long b0 = 0; b0 < N; b0 += chunk) {
+                const int nb = (int)std::min<long long>(chunk, N - b0);
+                if ((r = pmp_predict_maps(h, wq, wb, blk[c] + b0 * blk_bytes[c], PMP_IN_U8, nb, cqt, cbt, cdi, st.compute)))
+                    return r;
+                if ((r = pmp_qt_postprocess(h, cqt, nb, nullptr, qt8 + b0 * 64, st.compute))) return r;
+                for (int g = 0; g < ng; g++) {
+                    const int k = grp[g];
+                    uint8_t *d = dec(g);
+                    r = pmp_map2partition_ex(h, qt8 + b0 * 64, cbt, cdi, nb, c == 0 ? 1 : 2,
+                                             job.lamb ? job.lamb + 5 * res_q[k] : nullptr, cqt, h->near_tol,
+                                             d + b0 * 256, d + (size_t)nmax * 256 + b0 * 256,
+                                             (int8_t *)(d + (size_t)nmax * 512 + b0 * 768),
+                                             (uint32_t *)(o + off_flags[k]) + b0, st.compute);
+                    if (r) return r;
+                }
+            }
+            for (int g = 0; g < ng; g++) {
+                const int k = grp[g];
+                uint8_t *d = dec(g);
+                r = pmp_assemble_frames(h, d, d + (size_t)nmax * 256, qt8, (const int8_t *)(d + (size_t)nmax * 512), nf,
+                                        bh, bw, (int8_t *)(o + off_vals[k]), st.compute);
+                if (r) return r;
+                PMP_CUDA(cudaEventRecord(st.computed[s][k], st.compute));
+            }
         }
         if (job.text) {
             const int8_t *vals[RESULTS_MAX];
@@ -573,12 +629,12 @@ int run_windows(std::vector<Lane> &lanes, const WindowJob &job, pmp_report *tota
     return total->fp16_saturation_events ? saturation_error(total->fp16_saturation_events) : PMP_OK;
 }
 
-// pmp_predict_stream over `n` handles: wsets [n][n_qps][4], window k on hs[k % n].  caller >= 0 (the calling thread's
-// device): pmp_predict_stream_multi's messages, which name the handle, and its device rule, `caller` current in every
-// callback; -1: pmp_predict_stream's.
-int predict_stream(pmp_handle *const *hs, int n, int n_qps, const int *wsets, int frames, int width, int height,
-                   int sample_bytes, int window_frames, int outputs, pmp_read_cb read, pmp_write_cb write, void *user,
-                   pmp_report *report, int caller)
+// pmp_predict_stream over `n` handles: wsets [n][n_qps][4], lamb [n_qps][5] (checked by the caller) or nullptr, window
+// k on hs[k % n].  caller >= 0 (the calling thread's device): pmp_predict_stream_multi's messages, which name the handle,
+// and its device rule, `caller` current in every callback; -1: pmp_predict_stream's.
+int predict_stream(pmp_handle *const *hs, int n, int n_qps, const int *wsets, const double *lamb, int frames, int width,
+                   int height, int sample_bytes, int window_frames, int outputs, pmp_read_cb read, pmp_write_cb write,
+                   void *user, pmp_report *report, int caller)
 {
     const bool multi = caller >= 0;
     if (report) memset(report, 0, sizeof(*report));
@@ -651,6 +707,7 @@ int predict_stream(pmp_handle *const *hs, int n, int n_qps, const int *wsets, in
     PMP_CHECK_ARG((long long)wf * bpf < (1LL << 30) && (long long)wf * pmp_frame_values(bh, bw) <= TEXT_MAX_VALUES,
                   "too many blocks per window");
     job.n_qps = n_qps;
+    job.lamb = lamb;
     job.frames = frames;
     job.width = width;
     job.height = height;
@@ -681,6 +738,30 @@ int predict_stream(pmp_handle *const *hs, int n, int n_qps, const int *wsets, in
     pmp_report tot;
     const int rc = run_windows(lanes, job, &tot);
     if (report) *report = tot;
+    return rc;
+}
+
+// pmp_predict_stream_multi and pmp_predict_stream_ex: the handle list's checks, then predict_stream with the calling
+// thread's device current in the callbacks and restored on return.
+int predict_stream_handles(pmp_handle *const *handles, int n_handles, int n_rows, const int *wsets, const double *lamb,
+                           int frames, int width, int height, int sample_bytes, int window_frames, int outputs,
+                           pmp_read_cb read, pmp_write_cb write, void *user, pmp_report *report)
+{
+    PMP_CHECK_ARG(n_handles >= 1 && n_handles <= STREAM_HANDLES_MAX, "n_handles must be 1 to 16");
+    PMP_CHECK_ARG(handles != nullptr, "null handles");
+    for (int i = 0; i < n_handles; i++) {
+        if (!handles[i]) { set_error("bad argument: handles[%d] is null", i); return PMP_ERR_ARG; }
+        for (int j = 0; j < i; j++)
+            if (handles[j] == handles[i]) {
+                set_error("bad argument: handles[%d] is handles[%d]: every handle must be distinct", i, j);
+                return PMP_ERR_ARG;
+            }
+    }
+    int caller = 0;
+    PMP_CUDA(cudaGetDevice(&caller));
+    const int rc = predict_stream(handles, n_handles, n_rows, wsets, lamb, frames, width, height, sample_bytes,
+                                  window_frames, outputs, read, write, user, report, caller);
+    cudaSetDevice(caller);
     return rc;
 }
 
@@ -803,8 +884,8 @@ int pmp_predict_stream(pmp_handle *h, int n_qps, const int *wsets, int frames, i
                        pmp_report *report)
 {
     H_CHECK(h);
-    return predict_stream(&h, 1, n_qps, wsets, frames, width, height, sample_bytes, window_frames, outputs, read, write,
-                          user, report, -1);
+    return predict_stream(&h, 1, n_qps, wsets, nullptr, frames, width, height, sample_bytes, window_frames, outputs, read,
+                          write, user, report, -1);
 }
 
 int pmp_predict_stream_multi(pmp_handle *const *handles, int n_handles, int n_qps, const int *wsets, int frames,
@@ -812,22 +893,25 @@ int pmp_predict_stream_multi(pmp_handle *const *handles, int n_handles, int n_qp
                              pmp_write_cb write, void *user, pmp_report *report)
 {
     if (report) memset(report, 0, sizeof(*report));
-    PMP_CHECK_ARG(n_handles >= 1 && n_handles <= STREAM_HANDLES_MAX, "n_handles must be 1 to 16");
-    PMP_CHECK_ARG(handles != nullptr, "null handles");
-    for (int i = 0; i < n_handles; i++) {
-        if (!handles[i]) { set_error("bad argument: handles[%d] is null", i); return PMP_ERR_ARG; }
-        for (int j = 0; j < i; j++)
-            if (handles[j] == handles[i]) {
-                set_error("bad argument: handles[%d] is handles[%d]: every handle must be distinct", i, j);
+    return predict_stream_handles(handles, n_handles, n_qps, wsets, nullptr, frames, width, height, sample_bytes,
+                                  window_frames, outputs, read, write, user, report);
+}
+
+int pmp_predict_stream_ex(pmp_handle *const *handles, int n_handles, int n_rows, const int *wsets, const double *lamb,
+                          int frames, int width, int height, int sample_bytes, int window_frames, int outputs,
+                          pmp_read_cb read, pmp_write_cb write, void *user, pmp_report *report)
+{
+    if (report) memset(report, 0, sizeof(*report));
+    PMP_CHECK_ARG(n_rows >= 1 && n_rows <= 4, "n_rows must be 1 to 4");
+    for (int r = 0; lamb && r < n_rows; r++)
+        for (int k = 0; k < 5; k++)
+            if (!std::isfinite(lamb[5 * r + k])) {
+                set_error("bad argument: lamb[%d][%d] (row %d's lamb%d) is %g: every threshold must be finite", r, k, r,
+                          k + 1, lamb[5 * r + k]);
                 return PMP_ERR_ARG;
             }
-    }
-    int caller = 0;
-    PMP_CUDA(cudaGetDevice(&caller));
-    const int rc = predict_stream(handles, n_handles, n_qps, wsets, frames, width, height, sample_bytes, window_frames,
-                                  outputs, read, write, user, report, caller);
-    cudaSetDevice(caller);
-    return rc;
+    return predict_stream_handles(handles, n_handles, n_rows, wsets, lamb, frames, width, height, sample_bytes,
+                                  window_frames, outputs, read, write, user, report);
 }
 
 }  // extern "C"

@@ -2,7 +2,7 @@
 //
 //   pmp_predict --input SEQ.yuv --width W --height H --frames N [--bitDepth 8|10] [--ssRatio S] [--qps 22,27,32,37]
 //               --modelDir DIR --outDir DIR [--binaryOut] [--device D | --devices D,D,...] [--tcDtype fp16|bf16]
-//               [--chunk C] [--timing] [--stream]
+//               [--chunk C] [--timing] [--stream] [--lamb l1,l2,l3,l4,l5 ...]
 //
 // The weights are the exported .pmpw files (python -m pmp_vvc_tip2023_b200.export_weights): <comp>_Q_<qp>.pmpw and
 // <comp>_BD_<qp>.pmpw in --modelDir.  Frames are read as Inference_QBD.import_yuv420 reads them (every S-th frame, by
@@ -22,9 +22,16 @@
 // --devices D,D,... (with --stream) creates one handle per entry, each loading the same weight files, and makes one
 // pmp_predict_stream_multi call: window k runs on the (k mod n)-th handle while the files are written in frame order.
 // Entries may repeat (--devices 0,0: two handles on GPU 0).  A single entry without --stream is --device.
+//
+// --lamb l1,l2,l3,l4,l5 (with --stream, may be repeated) sets the decode thresholds lamb1..lamb5 of Map_to_Partition
+// (Map2Partition.py:100; the reference's defaults are 0.7,0.7,1.5,0.3,0.7) and makes one pmp_predict_stream_ex call
+// whose rows are every (setting, QP) pair, settings outermost, at most 4.  Settings of one QP share its net pass.  With
+// one --lamb the files go to --outDir under their usual names; with k > 1, setting i's (i = 0..k-1) go to
+// --outDir/lamb<i>/, and the tool prints which thresholds each directory holds.
 #include "pmp_b200.h"
 
 #include <chrono>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -39,6 +46,7 @@ struct Args {
     int width = 0, height = 0, frames = 0, bit_depth = 8, ss_ratio = 1, device = 0, chunk = 0;
     std::vector<int> qps{22, 27, 32, 37};
     std::vector<int> devices;       // --devices; empty: the one handle on --device
+    std::vector<std::vector<double> > lambs;      // --lamb settings, 5 thresholds each; empty: the defaults, no _ex call
     bool binary_out = false, bf16 = false, timing = false, stream = false, device_given = false;
 };
 
@@ -47,9 +55,26 @@ int usage(const char *msg)
     std::fprintf(stderr,
                  "pmp_predict: %s\nusage: pmp_predict --input SEQ.yuv --width W --height H --frames N [--bitDepth 8|10] "
                  "[--ssRatio S] [--qps 22,27,32,37] --modelDir DIR --outDir DIR [--binaryOut] [--device D | --devices D,D,...] "
-                 "[--tcDtype fp16|bf16] [--chunk C] [--timing] [--stream]\n",
+                 "[--tcDtype fp16|bf16] [--chunk C] [--timing] [--stream] [--lamb l1,l2,l3,l4,l5 ...]\n",
                  msg);
     return 2;
+}
+
+// "l1,l2,l3,l4,l5": exactly five finite decimal numbers
+bool parse_lamb(const std::string &v, std::vector<double> &out)
+{
+    out.clear();
+    for (size_t p = 0; p <= v.size();) {
+        size_t q = v.find(',', p);
+        if (q == std::string::npos) q = v.size();
+        const std::string x = v.substr(p, q - p);
+        char *end = nullptr;
+        const double d = std::strtod(x.c_str(), &end);
+        if (x.empty() || *end != 0 || !std::isfinite(d)) return false;
+        out.push_back(d);
+        p = q + 1;
+    }
+    return out.size() == 5;
 }
 
 bool parse(int argc, char **argv, Args &a, std::string &err)
@@ -84,6 +109,14 @@ bool parse(int argc, char **argv, Args &a, std::string &err)
                 p = q + 1;
             }
         }
+        else if (k == "--lamb") {
+            std::vector<double> l;
+            if (!parse_lamb(v, l)) {
+                err = "--lamb takes five comma-separated finite numbers l1,l2,l3,l4,l5, got '" + v + "'";
+                return false;
+            }
+            a.lambs.push_back(l);
+        }
         else if (k == "--chunk") a.chunk = std::atoi(v.c_str());
         else if (k == "--tcDtype") {
             if (v != "fp16" && v != "bf16") { err = "--tcDtype must be fp16 or bf16"; return false; }
@@ -110,6 +143,11 @@ bool parse(int argc, char **argv, Args &a, std::string &err)
     if (a.device_given && !a.devices.empty()) { err = "--device and --devices exclude each other"; return false; }
     if (a.devices.size() > 1 && !a.stream) { err = "--devices with more than one device needs --stream"; return false; }
     if (a.devices.size() > 16) { err = "--devices takes at most 16 entries"; return false; }
+    if (!a.lambs.empty() && !a.stream) { err = "--lamb needs --stream"; return false; }
+    if (a.lambs.size() * a.qps.size() > 4) {
+        err = "--lamb settings x --qps QPs make " + std::to_string(a.lambs.size() * a.qps.size()) + " rows, at most 4";
+        return false;
+    }
     return true;
 }
 
@@ -178,10 +216,10 @@ int saturated_exit(long long events)
     return 1;
 }
 
-std::string stem_of(const Args &a, const std::string &base, int qp, int c)
+std::string stem_of(const std::string &dir, const std::string &base, int qp, int c)
 {
     static const char *const comps[2] = {"Luma", "Chroma"};
-    return a.out_dir + "/" + base + "_" + comps[c] + "_QP" + std::to_string(qp) + "_PartitionMat";
+    return dir + "/" + base + "_" + comps[c] + "_QP" + std::to_string(qp) + "_PartitionMat";
 }
 
 // ---- --stream ------------------------------------------------------------------------------------------------------
@@ -190,7 +228,7 @@ struct Stream {
     FILE *in = nullptr;
     size_t ysz = 0, csz = 0;
     int sb = 1;
-    std::vector<FILE *> txt, bin;      // [2 * qp index + component]
+    std::vector<FILE *> txt, bin;      // [2 * row + component]
     std::string io_error;
 };
 
@@ -228,9 +266,21 @@ int stream_write(void *user, const pmp_window *w)
     return 0;
 }
 
-// hs: the one handle of pmp_predict_stream, or with --devices the handles of pmp_predict_stream_multi; wsets: [handle][qp][4]
+// hs: the one handle of pmp_predict_stream, or with --devices the handles of pmp_predict_stream_multi; wsets: [handle][qp][4].
+// With --lamb: the handles of one pmp_predict_stream_ex call whose rows are the (setting, QP) pairs.
 int run_stream(const Args &a, const std::vector<pmp_handle *> &hs, const std::vector<int> &wsets, const std::string &base)
 {
+    const int nset = a.lambs.empty() ? 1 : (int)a.lambs.size(), nq = (int)a.qps.size();
+    std::vector<int> row_qp;
+    std::vector<std::string> row_dir, set_dir;
+    for (int k = 0; k < nset; k++) {
+        set_dir.push_back(nset > 1 ? a.out_dir + "/lamb" + std::to_string(k) : a.out_dir);
+        for (int q = 0; q < nq; q++) {
+            row_qp.push_back(a.qps[q]);
+            row_dir.push_back(set_dir.back());
+        }
+    }
+    const int nrows = (int)row_qp.size();
     Stream st;
     st.a = &a;
     st.sb = a.bit_depth == 10 ? 2 : 1;
@@ -240,11 +290,13 @@ int run_stream(const Args &a, const std::vector<pmp_handle *> &hs, const std::ve
     st.in = std::fopen(a.input.c_str(), "rb");
     if (!st.in) { std::fprintf(stderr, "pmp_predict: cannot open %s\n", a.input.c_str()); return 1; }
     mkdir(a.out_dir.c_str(), 0777);      // an existing directory is fine; a failure shows when the files are opened
+    if (nset > 1)
+        for (const std::string &d : set_dir) mkdir(d.c_str(), 0777);
     std::vector<std::string> parts;
     bool ok = true;
-    for (size_t q = 0; q < a.qps.size() && ok; q++)
+    for (int r = 0; r < nrows && ok; r++)
         for (int c = 0; c < 2 && ok; c++) {
-            const std::string stem = stem_of(a, base, a.qps[q], c);
+            const std::string stem = stem_of(row_dir[r], base, row_qp[r], c);
             parts.push_back(stem + ".txt.part");
             FILE *t = std::fopen(parts.back().c_str(), "wb");
             FILE *b = nullptr;
@@ -266,7 +318,17 @@ int run_stream(const Args &a, const std::vector<pmp_handle *> &hs, const std::ve
         const auto t0 = std::chrono::steady_clock::now();
         const int window = a.chunk > 0 && bpf > 0 ? std::max(1, a.chunk / bpf) : 0;
         const int outputs = PMP_OUT_TEXT | (a.binary_out ? PMP_OUT_VALUES : 0), n = (int)hs.size();
-        if (a.devices.empty())
+        if (!a.lambs.empty()) {
+            std::vector<int> ws;            // [handle][setting][qp][4]
+            std::vector<double> lamb;       // [setting][qp][5]
+            for (int i = 0; i < n; i++)
+                for (int k = 0; k < nset; k++)
+                    ws.insert(ws.end(), wsets.begin() + 4 * nq * i, wsets.begin() + 4 * nq * (i + 1));
+            for (int k = 0; k < nset; k++)
+                for (int q = 0; q < nq; q++) lamb.insert(lamb.end(), a.lambs[k].begin(), a.lambs[k].end());
+            rc = pmp_predict_stream_ex(hs.data(), n, nrows, ws.data(), lamb.data(), nf, a.width, a.height, st.sb, window,
+                                       outputs, stream_read, stream_write, &st, &tot);
+        } else if (a.devices.empty())
             rc = pmp_predict_stream(hs[0], (int)a.qps.size(), wsets.data(), nf, a.width, a.height, st.sb, window, outputs,
                                     stream_read, stream_write, &st, &tot);
         else
@@ -274,7 +336,10 @@ int run_stream(const Args &a, const std::vector<pmp_handle *> &hs, const std::ve
                                           window, outputs, stream_read, stream_write, &st, &tot);
         const double ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
         const int wf = window > 0 ? window : std::max(1, bpf > 0 ? std::min(4800 / bpf, (nf + n - 1) / n) : 1);
-        if (a.timing && a.devices.empty())
+        if (a.timing && !a.lambs.empty())
+            std::printf("pmp_predict_stream_ex %.3f ms (%d frames, %d windows, %d handles, %d rows)\n", ms, nf,
+                        bpf > 0 ? (nf + wf - 1) / wf : 0, n, nrows);
+        else if (a.timing && a.devices.empty())
             std::printf("pmp_predict_stream %.3f ms (%d frames, %d windows)\n", ms, nf, bpf > 0 ? (nf + wf - 1) / wf : 0);
         else if (a.timing)
             std::printf("pmp_predict_stream_multi %.3f ms (%d frames, %d windows, %d handles)\n", ms, nf,
@@ -287,15 +352,19 @@ int run_stream(const Args &a, const std::vector<pmp_handle *> &hs, const std::ve
     }
     ok = ok && rc == PMP_OK && st.io_error.empty();
     if (ok) print_report(tot);
-    for (size_t q = 0; q < a.qps.size() && ok; q++)
+    for (int r = 0; r < nrows && ok; r++)
         for (int c = 0; c < 2 && ok; c++) {
-            const std::string stem = stem_of(a, base, a.qps[q], c);
+            const std::string stem = stem_of(row_dir[r], base, row_qp[r], c);
             ok = std::rename((stem + ".txt.part").c_str(), (stem + ".txt").c_str()) == 0;
             if (ok && a.binary_out) ok = std::rename((stem + ".bin.part").c_str(), (stem + ".bin").c_str()) == 0;
             else if (ok) std::remove((stem + ".bin").c_str());
             if (ok) std::printf("Save: %s.txt\n", stem.c_str());
             else std::fprintf(stderr, "pmp_predict: cannot rename %s.*.part\n", stem.c_str());
         }
+    for (int k = 0; k < nset && ok && !a.lambs.empty(); k++) {
+        const std::vector<double> &l = a.lambs[k];
+        std::printf("Thresholds of %s: lamb1..lamb5 = %g,%g,%g,%g,%g\n", set_dir[k].c_str(), l[0], l[1], l[2], l[3], l[4]);
+    }
     if (ok) return 0;
     for (const std::string &p : parts) std::remove(p.c_str());
     if (rc == PMP_ERR_STATE && tot.fp16_saturation_events) {
@@ -304,7 +373,7 @@ int run_stream(const Args &a, const std::vector<pmp_handle *> &hs, const std::ve
         return saturated_exit(tot.fp16_saturation_events);
     }
     if (!st.io_error.empty()) std::fprintf(stderr, "pmp_predict: %s\n", st.io_error.c_str());
-    if (rc != PMP_OK) return fail("pmp_predict_stream");
+    if (rc != PMP_OK) return fail(!a.lambs.empty() ? "pmp_predict_stream_ex" : "pmp_predict_stream");
     return 1;
 }
 
@@ -393,7 +462,7 @@ int main(int argc, char **argv)
     mkdir(a.out_dir.c_str(), 0777);      // an existing directory is fine; a failure shows when the files are written
     for (size_t q = 0; q < a.qps.size(); q++)
         for (int c = 0; c < 2; c++) {
-            const std::string stem = stem_of(a, base, a.qps[q], c);
+            const std::string stem = stem_of(a.out_dir, base, a.qps[q], c);
             std::printf("Save: %s.txt\n", stem.c_str());
             if (!write_text(stem + ".txt", out[2 * q + c])) return 1;
             if (a.binary_out) {
