@@ -177,7 +177,12 @@ int pmp_run_component(pmp_handle *h, int wset_q, int wset_msbd, int luma, const 
  * report (may be NULL): decode-flag counts of this call summed over both components (flags of pmp_map2partition;
  * near_threshold = bits 1..3, tight = bits 4..6) and the fp16 saturation events of this call (the sticky counter of
  * pmp_saturation_count is not reset).  Saturation events make the call return PMP_ERR_STATE: rerun with PMP_TC_BF16
- * (Inference_QBD.py:192-194 of this package refuses the same way). */
+ * (Inference_QBD.py:192-194 of this package refuses the same way).
+ * Repeated blocks: within a window, the nets run once per distinct cut block (68x68 luma, 3x34x34 chroma input bytes);
+ * byte-identical blocks get the first one's results (pmp_block_stats counts the work).  Values, flags and every report
+ * field but one are byte-identical to a run without reuse.  fp16_saturation_events (and the sticky counter) count the
+ * epilogue events of the blocks computed: a repeated block saturates exactly when its first occurrence does, so the
+ * PMP_ERR_STATE stop is unchanged, but the count is that of the distinct blocks. */
 typedef struct pmp_report {
     long long blocks, near_tie_blocks, near_threshold_blocks, near_threshold_blocks_tight, fp16_saturation_events;
 } pmp_report;
@@ -204,7 +209,10 @@ int pmp_predict_host(pmp_handle *h, const int wsets[4], const void *y, const voi
  * A non-zero return of either callback stops the call with PMP_ERR_ABORTED.  A window with fp16 saturation events is
  * still written; the call then stops with PMP_ERR_STATE (message as pmp_predict_host's).  *report (may be NULL) is the
  * sum over the windows written.  Every return, errors included, leaves no work queued and the handle usable.  Width or
- * height below 64 (zero blocks) returns PMP_OK without calling either callback. */
+ * height below 64 (zero blocks) returns PMP_OK without calling either callback.
+ * Repeated blocks within a window are computed once, as in pmp_predict_host: fp16_saturation_events counts the events of
+ * the distinct blocks, every other output is byte-identical to a run without reuse.  This holds for
+ * pmp_predict_stream_multi and pmp_predict_stream_ex too. */
 enum { PMP_OUT_VALUES = 1, PMP_OUT_TEXT = 2 };
 typedef struct pmp_window {
     int first_frame, frames, n_qps;
@@ -259,6 +267,13 @@ int pmp_predict_stream_ex(pmp_handle *const *handles, int n_handles, int n_rows,
                           int frames, int width, int height, int sample_bytes, int window_frames, int outputs,
                           pmp_read_cb read, pmp_write_cb write, void *user, pmp_report *report);
 
+/* pmp_block_stats: sticky per-handle counters of the window pipeline (pmp_predict_host, pmp_predict_stream(_multi,
+ * _ex)), summed over the net passes this handle ran since creation / the last reset: *blocks = the blocks of the passes'
+ * windows, *computed = the distinct blocks the nets actually ran on (a pass is one component of one window for one
+ * weight-set pair; rows sharing weight sets share it).  With 4 QPs, one window of N blocks with d distinct luma blocks
+ * adds 4N and 4d for luma.  Host counters: no synchronisation. */
+int pmp_block_stats(pmp_handle *h, long long *blocks, long long *computed, int reset);
+
 /* Self-test of the TC conv engine against the SIMT engine on random data (GPU).  Returns 0 and the
  * max-abs error in *max_err, or an error.  flags: bit0 ReLU, bit1 identity residual, bit2 attention product,
  * bit3 bf16 operands; kernel variants: bits 8..9 accumulator scheme of the single-CTA kernel (1 unstacked, 2 stacked),
@@ -285,6 +300,14 @@ int pmp_debug_conv(pmp_handle *h, const float *in, const float *w_host, const fl
  * (S = 64 luma / 32 chroma). */
 int pmp_debug_stem(pmp_handle *h, int wset, const void *blocks, int in_dtype, const float *qt, int B, float *out,
                    void *stream);
+
+/* Test hook: the window pipeline's grouping of repeated blocks (block_reuse.cu) on caller-supplied blocks.  blocks: n
+ * blocks of block_bytes bytes each (a positive multiple of 4; DEVICE, 4-byte aligned); rep: DEVICE int[n] receives, for
+ * every block i, the lowest index j with blocks j and i byte-identical.  hash_bits (0..64) keeps only that many low bits
+ * of the 64-bit fingerprints (0: every block collides), so that tests reach the byte comparison that confirms every
+ * fingerprint match.  *n_distinct_host (may be NULL): the number of i with rep[i] == i.  Synchronises the stream. */
+int pmp_debug_block_groups(pmp_handle *h, const uint8_t *blocks, int n, int block_bytes, int hash_bits, int *rep,
+                           int *n_distinct_host, void *stream);
 
 /* Debug/profiling aid: per-CTA barrier-stall cycle counters of the CTA-pair conv kernel (filled when the environment
  * variable PMP_TC_DBG has bit 6 set; 16 uint64 per CTA, see conv_tc.cu).  n = number of uint64 to copy (<= 2560). */

@@ -87,6 +87,8 @@ SIGNATURES = {
                                c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
     "pmp_debug_stem": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p]),
     "pmp_debug_tc_stalls": (c_int, [_P(ctypes.c_uint64), c_int]),
+    "pmp_block_stats": (c_int, [c_void_p, _P(ctypes.c_longlong), _P(ctypes.c_longlong), c_int]),
+    "pmp_debug_block_groups": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, _P(c_int), c_void_p]),
 }
 
 _lib = None
@@ -168,6 +170,13 @@ class Handle:
 
     def launch_count(self):
         return int(lib().pmp_launch_count(self._h))
+
+    def block_stats(self, reset=False):
+        """(blocks, computed): the blocks of the window pipeline's net passes on this handle and the distinct blocks the
+        nets ran on (repeated blocks in a window are computed once), since creation or the last reset."""
+        b, c = ctypes.c_longlong(), ctypes.c_longlong()
+        check(lib().pmp_block_stats(self._h, ctypes.byref(b), ctypes.byref(c), 1 if reset else 0))
+        return int(b.value), int(c.value)
 
     def profile(self, mode):
         check(lib().pmp_profile(self._h, mode))

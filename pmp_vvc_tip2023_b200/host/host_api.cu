@@ -2,8 +2,9 @@
 // pmp_weights_load (exported .pmpw weight files), pmp_predict_host (host planes in, host PartitionMat vectors out),
 // pmp_predict_stream (frames in through a callback, every QP's vectors and text out window by window),
 // pmp_predict_stream_multi (the same over several handles, windows in rotation), pmp_predict_stream_ex (the same with
-// decode thresholds per row) and pmp_format_texts (text_batch.cu), plus pmp_destroy, which releases this layer's staging
-// before the core handle teardown in csrc/api.cu.
+// decode thresholds per row), pmp_format_texts (text_batch.cu), pmp_block_stats and pmp_debug_block_groups (the reuse
+// of repeated blocks, block_reuse.cu), plus pmp_destroy, which releases this layer's staging before the core handle
+// teardown in csrc/api.cu.
 //
 // This layer only calls the core's entry points and internal functions; it lives outside csrc/ because bench.py ties
 // the committed ncu traffic summary (profiles/r*_traffic.json) to a hash of the csrc/ sources, and none of those kernels
@@ -163,20 +164,26 @@ int weights_load(Handle *h, const char *path, int *net_out, int *wset)
 
 // ---- the window pipeline of pmp_predict_host, pmp_predict_stream, pmp_predict_stream_multi and _ex ----------------
 // Per handle: a compute and a copy stream, their events, per window slot (double-buffered) pinned + device buffers for
-// the input planes and for the results (values, decode flags and, when asked for, text of every (row, component) pair,
-// the text byte counts and a snapshot of the saturation counter), and, used by the compute stream only, the cut blocks
-// and the work area of the per-window schedule (one chunk's float maps, the post-processed qt map and each row's decoded
-// integer maps).  Created on first use, grown to the largest window, released by pmp_destroy.
+// the input planes, the cut blocks and the results (values, decode flags and, when asked for, text of every (row,
+// component) pair, the text byte counts and a snapshot of the saturation counter), the grouping buffer (one grouping's
+// scratch, each slot's groups of both components, block_reuse.cu) with the distinct counts in pinned memory, and, used
+// by the compute stream only, the work area of the per-window schedule (one chunk's float maps, the post-processed qt
+// map, each row's decoded integer maps and flags, and for windows with repeats the compact blocks and one row expanded
+// to block order).  Created on first use, grown to the largest window, released by pmp_destroy.  The block counters of
+// pmp_block_stats live here too.
 constexpr int RESULTS_MAX = 8;      // 4 rows x 2 components
 constexpr int STREAM_HANDLES_MAX = 16;     // handles of one pmp_predict_stream_multi call
 
 struct HostStage {
     cudaStream_t compute = nullptr, copy = nullptr;
-    cudaEvent_t uploaded[2] = {}, cut[2] = {}, finished[2] = {}, downloaded[2] = {}, computed[2][RESULTS_MAX] = {};
+    cudaEvent_t uploaded[2] = {}, finished[2] = {}, downloaded[2] = {}, computed[2][RESULTS_MAX] = {};
     char *pin_in[2] = {}, *pin_out[2] = {}, *dev_in[2] = {}, *dev_out[2] = {};
-    uint8_t *dev_blocks = nullptr;
-    char *dev_work = nullptr;
-    size_t in_bytes = 0, out_bytes = 0, blocks_bytes = 0, work_bytes = 0;     // in, out: per slot
+    uint8_t *dev_blocks[2] = {};
+    char *dev_work = nullptr, *dev_group = nullptr;
+    int *pin_count = nullptr;               // [slot][component] distinct blocks of the slot's window
+    size_t in_bytes = 0, out_bytes = 0, blocks_bytes = 0, work_bytes = 0;     // in, out, blocks: per slot
+    long long group_cap = 0;                // blocks the grouping buffer holds
+    long long stat_blocks = 0, stat_computed = 0;       // pmp_block_stats
 };
 
 std::mutex g_stage_mu;
@@ -192,7 +199,7 @@ std::vector<cudaEvent_t *> events_of(HostStage &st)
 {
     std::vector<cudaEvent_t *> v;
     for (int s = 0; s < 2; s++) {
-        for (cudaEvent_t *e : {&st.uploaded[s], &st.cut[s], &st.finished[s], &st.downloaded[s]}) v.push_back(e);
+        for (cudaEvent_t *e : {&st.uploaded[s], &st.finished[s], &st.downloaded[s]}) v.push_back(e);
         for (cudaEvent_t &e : st.computed[s]) v.push_back(&e);
     }
     return v;
@@ -205,13 +212,28 @@ void free_buffers(HostStage &st)
         if (st.pin_out[s]) cudaFreeHost(st.pin_out[s]);
         if (st.dev_in[s]) cudaFree(st.dev_in[s]);
         if (st.dev_out[s]) cudaFree(st.dev_out[s]);
+        if (st.dev_blocks[s]) cudaFree(st.dev_blocks[s]);
         st.pin_in[s] = st.pin_out[s] = st.dev_in[s] = st.dev_out[s] = nullptr;
+        st.dev_blocks[s] = nullptr;
     }
-    if (st.dev_blocks) cudaFree(st.dev_blocks);
     if (st.dev_work) cudaFree(st.dev_work);
-    st.dev_blocks = nullptr;
-    st.dev_work = nullptr;
+    if (st.dev_group) cudaFree(st.dev_group);
+    st.dev_work = st.dev_group = nullptr;
     st.in_bytes = st.out_bytes = st.blocks_bytes = st.work_bytes = 0;
+    st.group_cap = 0;
+}
+
+// The grouping buffer for `cap` blocks.  Growing it waits for the device: work in flight may use the old one.
+int ensure_group(HostStage &st, long long cap)
+{
+    if (cap <= st.group_cap) return PMP_OK;
+    PMP_CUDA(cudaDeviceSynchronize());
+    if (st.dev_group) PMP_CUDA(cudaFree(st.dev_group));
+    st.dev_group = nullptr;
+    st.group_cap = 0;
+    PMP_CUDA(cudaMalloc((void **)&st.dev_group, group_bytes(cap)));
+    st.group_cap = cap;
+    return PMP_OK;
 }
 
 int ensure_stage(HostStage &st, size_t in_bytes, size_t out_bytes, size_t blocks_bytes, size_t work_bytes)
@@ -220,6 +242,7 @@ int ensure_stage(HostStage &st, size_t in_bytes, size_t out_bytes, size_t blocks
         PMP_CUDA(cudaStreamCreateWithFlags(&st.compute, cudaStreamNonBlocking));
         PMP_CUDA(cudaStreamCreateWithFlags(&st.copy, cudaStreamNonBlocking));
         for (cudaEvent_t *e : events_of(st)) PMP_CUDA(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
+        PMP_CUDA(cudaHostAlloc((void **)&st.pin_count, 4 * sizeof(int), cudaHostAllocDefault));
     }
     if (in_bytes <= st.in_bytes && out_bytes <= st.out_bytes && blocks_bytes <= st.blocks_bytes &&
         work_bytes <= st.work_bytes)
@@ -234,8 +257,8 @@ int ensure_stage(HostStage &st, size_t in_bytes, size_t out_bytes, size_t blocks
         PMP_CUDA(cudaHostAlloc((void **)&st.pin_out[s], out_bytes, cudaHostAllocDefault));
         PMP_CUDA(cudaMalloc((void **)&st.dev_in[s], in_bytes));
         PMP_CUDA(cudaMalloc((void **)&st.dev_out[s], out_bytes));
+        PMP_CUDA(cudaMalloc((void **)&st.dev_blocks[s], blocks_bytes));
     }
-    PMP_CUDA(cudaMalloc((void **)&st.dev_blocks, blocks_bytes));
     PMP_CUDA(cudaMalloc((void **)&st.dev_work, work_bytes));
     st.in_bytes = in_bytes;
     st.out_bytes = out_bytes;
@@ -258,6 +281,7 @@ void release_stage(const Handle *h)
     cudaDeviceSynchronize();
     free_buffers(st);
     if (!st.compute) return;
+    cudaFreeHost(st.pin_count);
     for (cudaEvent_t *e : events_of(st)) cudaEventDestroy(*e);
     cudaStreamDestroy(st.compute);
     cudaStreamDestroy(st.copy);
@@ -371,11 +395,16 @@ struct Lane {
 // uploads window k + n, downloads window k and writes window k - n, so each lane keeps both its window slots busy while
 // the host reads and writes in frame order; with one lane, window k+1 is filled and uploaded and window k-1 written
 // while window k computes.  Each lane's first window is computed as soon as it is uploaded, so that no device waits for
-// the other lanes' first reads.  Each window is cut into blocks once for all its results.  Per component, rows whose
-// (Q, MSBD) weight-set ids are equal share one net pass: per chunk of job.chunk blocks, pmp_predict_maps and
-// pmp_qt_postprocess run once and pmp_map2partition_ex once per row with the row's thresholds; then pmp_assemble_frames
-// runs once per row.  With one row per pass this is exactly the sequence of pmp_run_component.  The host waits only on
-// events of finished windows.  The device of a lane is made current before each of its CUDA calls; fill() and write()
+// the other lanes' first reads.  Each window is cut into blocks once for all its results, on the copy stream right after
+// its upload, and each component's blocks are grouped there (block_reuse.cu): the distinct count reaches pinned memory
+// behind the `uploaded` event, long before the compute stream gets to the window.  Per component, rows whose (Q, MSBD)
+// weight-set ids are equal share one net pass: per chunk of job.chunk blocks, pmp_predict_maps and pmp_qt_postprocess
+// run once and pmp_map2partition_ex once per row with the row's thresholds; then pmp_assemble_frames runs once per row.
+// With one row per pass this is exactly the sequence of pmp_run_component.  When a component's window holds repeated
+// blocks, the pass runs on its distinct blocks only: they are gathered into compact order first, and each row's decoded
+// maps, flags and the qt map are expanded back to block order before pmp_assemble_frames.  Without repeats the sequence
+// is the one above on the cut blocks.  The host waits only on events of finished windows and of uploads that finished
+// while an earlier window computed.  The device of a lane is made current before each of its CUDA calls; fill() and write()
 // may switch devices.  *total receives the sum of the reports of the windows written.  Every return leaves no work
 // queued on any lane.
 int run_windows(std::vector<Lane> &lanes, const WindowJob &job, pmp_report *total)
@@ -415,10 +444,14 @@ int run_windows(std::vector<Lane> &lanes, const WindowJob &job, pmp_report *tota
     const size_t off_nbytes = off, off_sat = off + 8 * RESULTS_MAX;
     const size_t blk_bytes[2] = {(size_t)68 * 68, (size_t)3 * 34 * 34};
     // the work area: one chunk's float maps (qt [64] | bt [768] | dire [768] f32 per block), the window's
-    // post-processed qt map [64] u8 per block, and per row of a shared net pass hor [256] | ver [256] | dire [768]
+    // post-processed qt map [64] u8 per block, per row of a shared net pass hor [256] | ver [256] | dire [768] and the
+    // flags [u32]; for windows with repeated blocks the compact blocks, the qt map and one row's maps in block order
     const int chunk = (int)std::min<long long>(job.chunk, nmax);
     const size_t maps_bytes = r256((size_t)chunk * (64 + 768 + 768) * sizeof(float)), qt8_bytes = r256((size_t)nmax * 64),
-                 row_bytes = r256((size_t)nmax * (256 + 256 + 768));
+                 dec_bytes = r256((size_t)nmax * (256 + 256 + 768)), row_bytes = dec_bytes + r256((size_t)nmax * 4),
+                 compact_bytes = r256((size_t)nmax * (comp_on[0] ? blk_bytes[0] : blk_bytes[1]));
+    const size_t off_rows = maps_bytes + qt8_bytes, off_compact = off_rows + (size_t)job.n_qps * row_bytes,
+                 off_qtx = off_compact + compact_bytes, off_expanded = off_qtx + qt8_bytes;
     const int nwin = (frames + wf - 1) / wf;
     if ((int)lanes.size() > nwin) lanes.resize(nwin);       // lanes without a window stay untouched
     const int n = (int)lanes.size();
@@ -429,8 +462,8 @@ int run_windows(std::vector<Lane> &lanes, const WindowJob &job, pmp_report *tota
         ln.st = &stage_of(h);
         rc = ensure_stage(*ln.st, (size_t)wf * in_frame, off_sat + 256,
                           (size_t)nmax * ((comp_on[0] ? blk_bytes[0] : 0) + (comp_on[1] ? blk_bytes[1] : 0)),
-                          maps_bytes + qt8_bytes + (size_t)job.n_qps * row_bytes);
-        if (rc) return rc;
+                          off_expanded + dec_bytes);
+        if (rc || (rc = ensure_group(*ln.st, nmax))) return rc;
         // The status word and the text status words exist before the loop (allocating them synchronises the device).
         // The activation arena grows inside the first window's pmp_predict_maps when a handle first sees this chunk
         // size; that synchronises the device once and leaves everything queued intact.
@@ -442,6 +475,9 @@ int run_windows(std::vector<Lane> &lanes, const WindowJob &job, pmp_report *tota
 
     auto win_frames = [&](int k) { return std::min(wf, frames - k * wf); };
     auto direct = [&](int f0, int i) -> int8_t * { return job.direct_out ? job.direct_out(f0, res_q[i], res_c[i]) : nullptr; };
+    auto blocks_of = [&](const HostStage &st, int s, int c) -> uint8_t * {
+        return !comp_on[c] ? nullptr : st.dev_blocks[s] + (c == 1 && comp_on[0] ? (size_t)nmax * blk_bytes[0] : 0);
+    };
 
     auto upload = [&](int k) -> int {
         Lane &ln = lanes[k % n];
@@ -450,7 +486,7 @@ int run_windows(std::vector<Lane> &lanes, const WindowJob &job, pmp_report *tota
         PMP_CUDA(cudaSetDevice(ln.h->device));
         if (j >= 2) {
             if (!job.direct_in) PMP_CUDA(cudaEventSynchronize(st.uploaded[s]));     // pin_in[s] free again
-            PMP_CUDA(cudaStreamWaitEvent(st.copy, st.cut[s], 0));                   // dev_in[s] read by the cut of j-2
+            PMP_CUDA(cudaStreamWaitEvent(st.copy, st.finished[s], 0));      // blocks and groups of slot s read by j-2
         }
         char *pin[3] = {nullptr, nullptr, nullptr};
         const char *src[3] = {nullptr, nullptr, nullptr};
@@ -461,6 +497,18 @@ int run_windows(std::vector<Lane> &lanes, const WindowJob &job, pmp_report *tota
         for (int p = 0; p < nplanes; p++)
             PMP_CUDA(cudaMemcpyAsync(st.dev_in[s] + in_off(p, nf), src[p], (size_t)nf * rows[p] * prow[p],
                                      cudaMemcpyHostToDevice, st.copy));
+        // cut and group on the copy stream, so that the distinct counts are on the host before compute(k) needs them
+        const char *d = st.dev_in[s];
+        r = cut_blocks(ln.h, d, chroma ? d + in_off(1, nf) : nullptr, chroma ? d + in_off(2, nf) : nullptr,
+                       job.sample_bytes, nf, job.width, job.height, blocks_of(st, s, 0), blocks_of(st, s, 1), st.copy);
+        if (r) return r;
+        for (int c = 0; c < 2; c++)
+            if (comp_on[c] && (r = group_blocks(ln.h, st.dev_group, st.group_cap, blocks_of(st, s, c), nf * bpf,
+                                                (int)blk_bytes[c], 64, nullptr, groups_of(st.dev_group, st.group_cap, s, c),
+                                                st.copy)))
+                return r;
+        PMP_CUDA(cudaMemcpyAsync(st.pin_count + 2 * s, groups_of(st.dev_group, st.group_cap, s, 0).count, 2 * sizeof(int),
+                                 cudaMemcpyDeviceToHost, st.copy));
         PMP_CUDA(cudaEventRecord(st.uploaded[s], st.copy));
         return PMP_OK;
     };
@@ -472,17 +520,13 @@ int run_windows(std::vector<Lane> &lanes, const WindowJob &job, pmp_report *tota
         PMP_CUDA(cudaSetDevice(h->device));
         PMP_CUDA(cudaStreamWaitEvent(st.compute, st.uploaded[s], 0));
         if (j >= 2) PMP_CUDA(cudaStreamWaitEvent(st.compute, st.downloaded[s], 0));   // dev_out[s] read by j-2
-        const char *d = st.dev_in[s];
+        PMP_CUDA(cudaEventSynchronize(st.uploaded[s]));         // the distinct counts; in steady state long recorded
         char *o = st.dev_out[s];
-        uint8_t *blk[2] = {comp_on[0] ? st.dev_blocks : nullptr,
-                           comp_on[1] ? st.dev_blocks + (comp_on[0] ? (size_t)nmax * blk_bytes[0] : 0) : nullptr};
-        int r = cut_blocks(h, d, chroma ? d + in_off(1, nf) : nullptr, chroma ? d + in_off(2, nf) : nullptr,
-                           job.sample_bytes, nf, job.width, job.height, blk[0], blk[1], st.compute);
-        if (r) return r;
-        PMP_CUDA(cudaEventRecord(st.cut[s], st.compute));
         const long long N = (long long)nf * bpf;
         float *cqt = (float *)st.dev_work, *cbt = cqt + (size_t)chunk * 64, *cdi = cbt + (size_t)chunk * 768;
-        uint8_t *qt8 = (uint8_t *)st.dev_work + maps_bytes;
+        uint8_t *qt8 = (uint8_t *)st.dev_work + maps_bytes, *compact = (uint8_t *)st.dev_work + off_compact,
+                *qtx = (uint8_t *)st.dev_work + off_qtx, *expanded = (uint8_t *)st.dev_work + off_expanded;
+        int r = PMP_OK;
         bool done[RESULTS_MAX] = {};
         for (int i = 0; i < nres; i++) {
             if (done[i]) continue;
@@ -496,10 +540,22 @@ int run_windows(std::vector<Lane> &lanes, const WindowJob &job, pmp_report *tota
                     done[j] = true;
                 }
             }
-            auto dec = [&](int g) { return (uint8_t *)st.dev_work + maps_bytes + qt8_bytes + (size_t)g * row_bytes; };
-            for (long long b0 = 0; b0 < N; b0 += chunk) {
-                const int nb = (int)std::min<long long>(chunk, N - b0);
-                if ((r = pmp_predict_maps(h, wq, wb, blk[c] + b0 * blk_bytes[c], PMP_IN_U8, nb, cqt, cbt, cdi, st.compute)))
+            auto dec = [&](int g) { return (uint8_t *)st.dev_work + off_rows + (size_t)g * row_bytes; };
+            auto dec_flags = [&](int g) { return (uint32_t *)(dec(g) + dec_bytes); };
+            // the net pass runs on the nd distinct blocks: in place without repeats, else gathered into compact order
+            const Groups grps = groups_of(st.dev_group, st.group_cap, s, c);
+            const int nd = st.pin_count[2 * s + c];
+            const bool reuse = nd < N;
+            const uint8_t *src = blocks_of(st, s, c);
+            if (reuse) {
+                if ((r = gather_blocks(h, src, grps.distinct, nd, (int)blk_bytes[c], compact, st.compute))) return r;
+                src = compact;
+            }
+            st.stat_blocks += N;
+            st.stat_computed += nd;
+            for (long long b0 = 0; b0 < nd; b0 += chunk) {
+                const int nb = (int)std::min<long long>(chunk, nd - b0);
+                if ((r = pmp_predict_maps(h, wq, wb, src + b0 * blk_bytes[c], PMP_IN_U8, nb, cqt, cbt, cdi, st.compute)))
                     return r;
                 if ((r = pmp_qt_postprocess(h, cqt, nb, nullptr, qt8 + b0 * 64, st.compute))) return r;
                 for (int g = 0; g < ng; g++) {
@@ -509,15 +565,22 @@ int run_windows(std::vector<Lane> &lanes, const WindowJob &job, pmp_report *tota
                                              job.lamb ? job.lamb + 5 * res_q[k] : nullptr, cqt, h->near_tol,
                                              d + b0 * 256, d + (size_t)nmax * 256 + b0 * 256,
                                              (int8_t *)(d + (size_t)nmax * 512 + b0 * 768),
-                                             (uint32_t *)(o + off_flags[k]) + b0, st.compute);
+                                             (reuse ? dec_flags(g) : (uint32_t *)(o + off_flags[k])) + b0, st.compute);
                     if (r) return r;
                 }
             }
             for (int g = 0; g < ng; g++) {
                 const int k = grp[g];
                 uint8_t *d = dec(g);
-                r = pmp_assemble_frames(h, d, d + (size_t)nmax * 256, qt8, (const int8_t *)(d + (size_t)nmax * 512), nf,
-                                        bh, bw, (int8_t *)(o + off_vals[k]), st.compute);
+                if (reuse) {        // this row's maps and flags (and once the qt map) back to block order
+                    r = expand_blocks(h, grps.slot, (int)N, nmax, d, expanded, dec_flags(g), (uint32_t *)(o + off_flags[k]),
+                                      g == 0 ? qt8 : nullptr, qtx, st.compute);
+                    if (r) return r;
+                    d = expanded;
+                }
+                r = pmp_assemble_frames(h, d, d + (size_t)nmax * 256, reuse ? qtx : qt8,
+                                        (const int8_t *)(d + (size_t)nmax * 512), nf, bh, bw, (int8_t *)(o + off_vals[k]),
+                                        st.compute);
                 if (r) return r;
                 PMP_CUDA(cudaEventRecord(st.computed[s][k], st.compute));
             }
@@ -912,6 +975,41 @@ int pmp_predict_stream_ex(pmp_handle *const *handles, int n_handles, int n_rows,
             }
     return predict_stream_handles(handles, n_handles, n_rows, wsets, lamb, frames, width, height, sample_bytes,
                                   window_frames, outputs, read, write, user, report);
+}
+
+int pmp_block_stats(pmp_handle *h, long long *blocks, long long *computed, int reset)
+{
+    H_CHECK(h);
+    PMP_CHECK_ARG(blocks && computed, "null pointer");
+    HostStage &st = stage_of(h);
+    *blocks = st.stat_blocks;
+    *computed = st.stat_computed;
+    if (reset) st.stat_blocks = st.stat_computed = 0;
+    return PMP_OK;
+}
+
+int pmp_debug_block_groups(pmp_handle *h, const uint8_t *blocks, int n, int block_bytes, int hash_bits, int *rep,
+                           int *n_distinct_host, void *stream)
+{
+    H_CHECK(h);
+    if (n_distinct_host) *n_distinct_host = 0;
+    PMP_CHECK_ARG(n >= 0 && n < (1 << 30), "n must be 0 to 2^30 - 1");
+    PMP_CHECK_ARG(block_bytes > 0 && block_bytes % 4 == 0, "block_bytes must be a positive multiple of 4");
+    PMP_CHECK_ARG(hash_bits >= 0 && hash_bits <= 64, "hash_bits must be 0 to 64");
+    if (n == 0) return PMP_OK;
+    PMP_CHECK_ARG(blocks && rep, "null pointer");
+    PMP_CHECK_ARG(((uintptr_t)blocks & 3) == 0, "blocks must be 4-byte aligned");
+    HostStage &st = stage_of(h);
+    int rc = ensure_group(st, n);
+    if (rc) return rc;
+    cudaStream_t s = (cudaStream_t)stream;
+    const Groups g = groups_of(st.dev_group, st.group_cap, 0, 0);
+    if ((rc = group_blocks(h, st.dev_group, st.group_cap, blocks, n, block_bytes, hash_bits, rep, g, s))) return rc;
+    int nd = 0;
+    PMP_CUDA(cudaMemcpyAsync(&nd, g.count, sizeof(int), cudaMemcpyDeviceToHost, s));
+    PMP_CUDA(cudaStreamSynchronize(s));
+    if (n_distinct_host) *n_distinct_host = nd;
+    return PMP_OK;
 }
 
 }  // extern "C"

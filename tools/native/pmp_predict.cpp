@@ -28,6 +28,9 @@
 // whose rows are every (setting, QP) pair, settings outermost, at most 4.  Settings of one QP share its net pass.  With
 // one --lamb the files go to --outDir under their usual names; with k > 1, setting i's (i = 0..k-1) go to
 // --outDir/lamb<i>/, and the tool prints which thresholds each directory holds.
+//
+// After the run the tool prints the "Decode report:" line and a "Block reuse:" line: within a window the library runs the
+// nets once per distinct block (pmp_block_stats), and the line says on how many of the blocks they ran.
 #include "pmp_b200.h"
 
 #include <chrono>
@@ -209,6 +212,21 @@ void print_report(const pmp_report &tot)
                 0.01 * near_tol, tot.fp16_saturation_events);
 }
 
+// The nets' work summed over the handles (pmp_block_stats): blocks computed of the blocks of every net pass.
+void print_reuse(const std::vector<pmp_handle *> &hs)
+{
+    long long blocks = 0, computed = 0;
+    for (pmp_handle *h : hs) {
+        long long b = 0, c = 0;
+        if (pmp_block_stats(h, &b, &c, 0) == PMP_OK) {
+            blocks += b;
+            computed += c;
+        }
+    }
+    std::printf("Block reuse: the nets ran on %lld of %lld blocks (%.1f %%)\n", computed, blocks,
+                blocks ? 100.0 * computed / blocks : 100.0);
+}
+
 int saturated_exit(long long events)
 {
     std::fprintf(stderr, "pmp_predict: activations left the fp16 range (%lld events): results are clamped; rerun with "
@@ -351,7 +369,10 @@ int run_stream(const Args &a, const std::vector<pmp_handle *> &hs, const std::ve
         if (st.bin[i] && std::fclose(st.bin[i]) != 0) st.io_error = "write error";
     }
     ok = ok && rc == PMP_OK && st.io_error.empty();
-    if (ok) print_report(tot);
+    if (ok) {
+        print_report(tot);
+        print_reuse(hs);
+    }
     for (int r = 0; r < nrows && ok; r++)
         for (int c = 0; c < 2 && ok; c++) {
             const std::string stem = stem_of(row_dir[r], base, row_qp[r], c);
@@ -455,8 +476,9 @@ int main(int argc, char **argv)
         tot.near_threshold_blocks_tight += r.near_threshold_blocks_tight;
         tot.fp16_saturation_events += r.fp16_saturation_events;
     }
-    pmp_destroy(h);
     print_report(tot);
+    print_reuse(hs);
+    pmp_destroy(h);
     if (saturated) return saturated_exit(tot.fp16_saturation_events);
 
     mkdir(a.out_dir.c_str(), 0777);      // an existing directory is fine; a failure shows when the files are written
